@@ -2,7 +2,12 @@
 """bench.py — BASELINE.json's metric on BASELINE.json's configs, one JSON line on stdout.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg2|cfg4|cfg5|strong|k2]
+                  [--dump-outputs DIR]
   (N > 1: launched by torchrun, one rank per GPU; RANK / LOCAL_RANK / WORLD_SIZE from the env)
+
+--dump-outputs DIR (cfg2 / strong): after the timed steps, rank 0 writes what its last timed CorrelateScan returned for
+its batch as DIR/{response,pose,covariance,status,tie_count}.npy (float64; status and tie counts are integers held
+exactly).  The inputs are seeded, so two builds run with the same arguments can be compared output for output.
 
 --workload cfg2 (default, the headline; config.workload = "cfg2"): B = 1024 synthetic 1081-beam scans per GPU (Hokuyo
 UTM-30LX model), each matched against its own 0.05 m correlation grid (one base scan, 20.05 m x 20.05 m ROI) with a direct
@@ -74,7 +79,20 @@ def parse():
     ap.add_argument("--quick", action="store_true", help="smaller secondary sections (development)")
     ap.add_argument("--nodes", type=int, default=5000, help="cfg5: key frames of the trajectory")
     ap.add_argument("--min-seconds", type=float, default=0.0, help="repeat the timed steps until at least this long")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's results as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload not in ("cfg2", "strong")):
+        ap.error("--dump-outputs covers the cfg2 / strong CorrelateScan path of --impl ours")
+    return args
+
+
+def dump_outputs(directory, out):
+    """The arrays correlate_scan returned (response, pose, covariance, status, tie_count) as float64 .npy files."""
+    os.makedirs(directory, exist_ok=True)
+    for name, a in zip(("response", "pose", "covariance", "status", "tie_count"), out):
+        np.save(os.path.join(directory, name + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 def cfg2_config(B, world):
@@ -922,8 +940,7 @@ def workload_cfg2(ctx, args, strong=False):
     m.add_scans(bran, bpos)
     m.sync()
     for _ in range(args.warmup):
-        out = m.correlate_scan(poses, se)
-    assert (out[3] == 0).all() and m.last_timing()["path"] == 2
+        m.correlate_scan(poses, se)
     sampler = ClockSampler(local)
     sampler.start()
     time.sleep(0.3)
@@ -937,6 +954,9 @@ def workload_cfg2(ctx, args, strong=False):
 
     ms_max, per_rank_ms, steps_done = ctx.timed(step, args.steps, args.min_seconds)
     out = last["out"]
+    assert (out[3] == 0).all() and m.last_timing()["path"] == 2
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out)
     empty_frac = m.last_stats()["empty_window_frac"]
     total = (args.batch if strong else world * B)
     value = total * steps_done / (ms_max * 1e-3)

@@ -6,6 +6,8 @@ import os
 import subprocess
 import sys
 
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -30,3 +32,24 @@ def test_product_arm_fails_loudly_without_a_gpu():
     p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "1", "--warmup", "1"], cwd=ROOT,
                        capture_output=True, text=True, timeout=300)
     assert p.returncode != 0 and p.stdout.strip() == "" and "no CUDA device" in p.stderr
+
+
+@pytest.mark.gpu
+def test_dump_outputs_writes_the_last_timed_step(tmp_path):
+    """--dump-outputs: the CorrelateScan results of the last timed step, float64, one row per match of the batch; --steps
+    sets the number of timed steps; the same seeded inputs give the same outputs run after run."""
+    import numpy as np
+    outs = []
+    for run in ("a", "b"):
+        p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "3", "--warmup", "0", "--batch", "16",
+                            "--no-k2", "--no-cpu-baseline", "--quick", "--dump-outputs", str(tmp_path / run)],
+                           cwd=ROOT, capture_output=True, text=True, timeout=600)
+        assert p.returncode == 0, p.stderr[-2000:]
+        d = json.loads(p.stdout)
+        assert d["steps"] == 3 and d["multi_gpu_exact"]["ok"]
+        got = {n: np.load(tmp_path / run / f"{n}.npy") for n in ("response", "pose", "covariance", "status", "tie_count")}
+        assert all(a.dtype == np.float64 for a in got.values())
+        assert got["response"].shape == (16,) and got["pose"].shape == (16, 3) and got["covariance"].shape == (16, 3, 3)
+        assert (got["status"] == 0).all() and (got["tie_count"] >= 1).all() and (got["response"] > 0).all()
+        outs.append(got)
+    assert all(np.array_equal(outs[0][n], outs[1][n]) for n in outs[0])

@@ -1,6 +1,7 @@
 """GPU tests of the lesson6 front end through the C ABI (b2s_mapper_*): every MatchScan on the CUDA matcher, near-chain
 and loop-candidate matches batched.  Checked against the reference Mapper's golden output (tests/golden/karto_mapper.npz)
-and, where the reference build travelled with the repo, against the live reference with the same back end plugged in."""
+and against the reference Mapper with the same back end plugged in (its recorded answers where the reference build is
+absent: tests/reference_replay.py)."""
 import os
 
 import numpy as np
@@ -51,12 +52,11 @@ def test_mapper_cuda_multi_robot_vs_reference_golden(pkg):
     m.close()
 
 
-@pytest.mark.skipif(not ref.available(), reason="oracle/_ref/libkarto_ref.so did not travel")
-def test_mapper_cuda_vs_live_reference_with_back_end(pkg):
+def test_mapper_cuda_vs_live_reference_with_back_end(pkg, reference):
     MP, abi = pkg.load("mapper"), pkg.abi
     laser, prm, true, odom, ranges = mc.workload(pkg, 5, 130, drift=(0.01, 0.008, 0.004))
-    g1, g2 = MP.PoseGraph(), MP.PoseGraph()
-    r = ref.RefMapper(prm, laser)
+    g1, g2 = reference.new(MP.PoseGraph), MP.PoseGraph()
+    r = reference.new(ref.RefMapper, prm, laser)
     r.set_scan_solver(g1.as_scan_solver())
     m = MP.Mapper(prm, abi.laser_from(laser))
     m.set_scan_solver(g2.as_scan_solver())

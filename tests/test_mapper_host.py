@@ -1,5 +1,6 @@
 """CPU tests of the mapper's HOST logic (karto_mapper.cu: key-frame gate, running window, graph edges, near chains,
-loop-closure candidates, ScanSolver plug-in) against the UNMODIFIED reference karto::Mapper (oracle/_ref/libkarto_ref.so).
+loop-closure candidates, ScanSolver plug-in) against the UNMODIFIED reference karto::Mapper (oracle/_ref/libkarto_ref.so,
+or its recorded answers where that build is absent: tests/reference_replay.py).
 No GPU here: the product's matcher plug-in point is served by the CPU restatement's MatchScan (tests only), the
 reference uses its own ScanMatcher — so every difference would come from the graph / pose logic under test."""
 import os
@@ -11,7 +12,6 @@ from oracle import port, ref
 import mapper_cases as mc
 
 G = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
-live = pytest.mark.skipif(not ref.available(), reason="oracle/_ref/libkarto_ref.so not built")
 
 
 def compare(r, m, tol=1e-9):
@@ -22,14 +22,13 @@ def compare(r, m, tol=1e-9):
     assert np.abs(dr - dm).max() <= tol and np.abs(cr - cm).max() <= tol
 
 
-@live
-def test_mapper_matches_reference_without_back_end(pkg):
+def test_mapper_matches_reference_without_back_end(pkg, reference):
     """150 scans, 3 laps: sequential matches against the running window, near-chain links (batched), loop closures
     accepted without a solver (the lesson6 indoor yaml: use_back_end false)."""
     MP, abi = pkg.load("mapper"), pkg.abi
     laser, prm, true, odom, ranges = mc.workload(pkg, 3, 150)
     al = abi.laser_from(laser)
-    r = ref.RefMapper(prm, laser)
+    r = reference.new(ref.RefMapper, prm, laser)
     m = MP.Mapper(prm, al, match_fn=port.mapper_match_hook(prm, al))
     fr, cr = mc.run(r, odom, ranges)
     fm, cm = mc.run(m, odom, ranges)
@@ -44,15 +43,14 @@ def test_mapper_matches_reference_without_back_end(pkg):
     r.close(), m.close()
 
 
-@live
-def test_mapper_with_scan_solver_plugin(pkg):
+def test_mapper_with_scan_solver_plugin(pkg, reference):
     """The same back end (the library's pose-graph optimiser, one instance per side) plugged into the reference Mapper
     through karto::ScanSolver and into ours through b2s_scan_solver: corrected poses agree after every loop closure."""
     MP, abi = pkg.load("mapper"), pkg.abi
     laser, prm, true, odom, ranges = mc.workload(pkg, 5, 130, drift=(0.01, 0.008, 0.004))
     al = abi.laser_from(laser)
-    g1, g2 = MP.PoseGraph(), MP.PoseGraph()
-    r = ref.RefMapper(prm, laser)
+    g1, g2 = reference.new(MP.PoseGraph), MP.PoseGraph()
+    r = reference.new(ref.RefMapper, prm, laser)
     r.set_scan_solver(g1.as_scan_solver())
     m = MP.Mapper(prm, al, match_fn=port.mapper_match_hook(prm, al))
     m.set_scan_solver(g2.as_scan_solver())
@@ -67,14 +65,13 @@ def test_mapper_with_scan_solver_plugin(pkg):
     r.close(), m.close()
 
 
-@live
-def test_mapper_key_frame_gate(pkg):
+def test_mapper_key_frame_gate(pkg, reference):
     """Mapper::HasMovedEnough (Mapper.cpp:2087-2119): travel distance, heading and time interval."""
     MP, abi = pkg.load("mapper"), pkg.abi
     laser, prm, true, odom, ranges = mc.workload(pkg, 7, 12)
     prm.minimum_time_interval = 5.0
     al = abi.laser_from(laser)
-    r = ref.RefMapper(prm, laser)
+    r = reference.new(ref.RefMapper, prm, laser)
     m = MP.Mapper(prm, al, match_fn=port.mapper_match_hook(prm, al))
     seq = [(0, 0.0), (0, 1.0), (1, 2.0), (1, 3.0), (1, 9.0), (2, 9.5)]  # (pose index, time): repeats are rejected
     tiny = odom[2] + np.array([0.05, 0.0, 0.02])
@@ -91,9 +88,8 @@ def test_mapper_key_frame_gate(pkg):
     r.close(), m.close()
 
 
-@live
 @pytest.mark.parametrize("prefixes,solver,seed", [(("a_robot", "z_robot"), False, 3), (("z_robot", "a_robot"), True, 7)])
-def test_mapper_multi_robot_matches_reference(pkg, prefixes, solver, seed):
+def test_mapper_multi_robot_matches_reference(pkg, reference, prefixes, solver, seed):
     """MapperSensorManager semantics with three sensors (Mapper.cpp:45-100, 920-952, 1170-1275, 1333-1394, 2063-2070):
     a sensor's first scan is matched against all scans of the other sensors and linked to their first scans, near
     chains follow the near scan's own sensor, loop closures are searched per sensor in NAME order — the two extra
@@ -101,10 +97,10 @@ def test_mapper_multi_robot_matches_reference(pkg, prefixes, solver, seed):
     MP, abi = pkg.load("mapper"), pkg.abi
     laser, prm, true, odom, ranges = mc.workload(pkg, seed, 150, drift=mc.FLEET_DRIFT)
     al = abi.laser_from(laser)
-    r = ref.RefMapper(prm, laser)
+    r = reference.new(ref.RefMapper, prm, laser)
     m = MP.Mapper(prm, al, match_fn=port.mapper_match_hook(prm, al))
     if solver:
-        g1, g2 = MP.PoseGraph(), MP.PoseGraph()
+        g1, g2 = reference.new(MP.PoseGraph), MP.PoseGraph()
         r.set_scan_solver(g1.as_scan_solver())
         m.set_scan_solver(g2.as_scan_solver())
     ref_ids = [0] + [r.add_sensor(p) for p in prefixes]
@@ -252,8 +248,7 @@ def test_pose_graph_sparse_ldlt_reaches_the_least_squares_optimum(pkg):
     g.close()
 
 
-@live
-def test_mapper_with_dropouts(pkg):
+def test_mapper_with_dropouts(pkg, reference):
     """1 % of the readings replaced by NaN / 0.0 (below min range): unfiltered points, barycenters and every decision
     still agree with the reference exactly."""
     MP, abi = pkg.load("mapper"), pkg.abi
@@ -263,7 +258,7 @@ def test_mapper_with_dropouts(pkg):
     for k, (i, j) in enumerate(np.argwhere(rng.random(r2.shape) < 0.01)):
         r2[i, j] = np.nan if k % 2 == 0 else 0.0
     al = abi.laser_from(laser)
-    r = ref.RefMapper(prm, laser)
+    r = reference.new(ref.RefMapper, prm, laser)
     m = MP.Mapper(prm, al, match_fn=port.mapper_match_hook(prm, al))
     fr, _ = mc.run(r, odom, r2)
     fm, _ = mc.run(m, odom, r2)
@@ -272,8 +267,7 @@ def test_mapper_with_dropouts(pkg):
     r.close(), m.close()
 
 
-@live
-def test_mapper_singular_covariance_is_an_error_where_the_reference_asserts(pkg, tmp_path):
+def test_mapper_singular_covariance_is_an_error_where_the_reference_asserts(pkg, reference, tmp_path):
     """ComputeWeightedMean inverts the link covariances with Matrix3::Inverse, which ASSERTS when |det| <= 1e-14
     (Karto.h:2445-2453; the catkin build keeps asserts).  On this seeded stream the reference aborts at some scan; ours
     must report B2S_ERR_BAD_STATE at the same scan instead of continuing with garbage."""
@@ -286,11 +280,14 @@ def test_mapper_singular_covariance_is_an_error_where_the_reference_asserts(pkg,
             "laser, prm, true, odom, ranges = mc.workload(pkg, 9, 70)\nr = ref.RefMapper(prm, laser)\n"
             "for i in range(70):\n    print(i, flush=True)\n    r.process(ranges[i], odom[i], 0.1 * i)\nprint('done', flush=True)\n"
             % (os.path.dirname(os.path.dirname(os.path.abspath(__file__))), os.path.dirname(os.path.abspath(__file__))))
-    out = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=300)
-    lines = out.stdout.split()
-    assert out.returncode != 0 and lines[-1] != "done" and "Assertion" in out.stderr
-    ref_fail = int(lines[-1])
     laser, prm, true, odom, ranges = mc.workload(pkg, 9, 70)
+
+    def reference_failing_scan(*workload):  # runs `code`; the workload is passed to tie the recording to it
+        out = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=300)
+        lines = out.stdout.split()
+        assert out.returncode != 0 and lines[-1] != "done" and "Assertion" in out.stderr
+        return int(lines[-1])
+    ref_fail = reference.call("scan at which the reference Mapper asserts", reference_failing_scan, prm, laser, odom, ranges)
     al = abi.laser_from(laser)
     m = MP.Mapper(prm, al, match_fn=port.mapper_match_hook(prm, al))
     ours_fail = None
@@ -305,15 +302,18 @@ def test_mapper_singular_covariance_is_an_error_where_the_reference_asserts(pkg,
     m.close()
 
 
-@live
-def test_mapper_default_params_equal_the_reference(pkg):
+def test_mapper_default_params_equal_the_reference(pkg, reference):
     """b2s_mapper_default_params vs the values a fresh karto::Mapper holds (Mapper::InitializeParameters)."""
     import ctypes as C
     MP = pkg.load("mapper")
     ours = MP.default_params(12.0)
-    theirs = MP.MapperParams()
-    ref._lib(False).ref_mapper_default_params(C.byref(theirs))
-    theirs.sequential.range_threshold = theirs.loop.range_threshold = 12.0  # comes from the laser, not from the Mapper
+
+    def reference_defaults():
+        theirs = MP.MapperParams()
+        ref._lib(False).ref_mapper_default_params(C.byref(theirs))
+        theirs.sequential.range_threshold = theirs.loop.range_threshold = 12.0  # comes from the laser, not the Mapper
+        return flat(theirs)
+
     def flat(p):
         out = {}
         for name, _ in p._fields_:
@@ -323,7 +323,7 @@ def test_mapper_default_params_equal_the_reference(pkg):
             else:
                 out[name] = v
         return out
-    a, b = flat(ours), flat(theirs)
+    a, b = flat(ours), reference.call("karto::Mapper default parameters", reference_defaults)
     assert a.keys() == b.keys()
     for k in a:
         assert a[k] == b[k], (k, a[k], b[k])

@@ -4,9 +4,9 @@ test_oracle_hector_reference.py)."""
 import os
 
 import numpy as np
-import pytest
 
 from oracle import port, ref_gmapping as rg
+from reference_replay import same
 
 G = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
@@ -25,26 +25,32 @@ def test_gmapping_golden():
         assert np.array_equal(ax[ys, xs], g[f"c{k}_acc_x"]) and np.array_equal(ay[ys, xs], g[f"c{k}_acc_y"])
 
 
-@pytest.mark.skipif(not rg.available(), reason="oracle/_ref/libgmapping_ref.so not built")
-def test_gmapping_live(pkg):
+def test_gmapping_live(pkg, reference):
+    """Against the reference's grid headers (oracle/_ref/libgmapping_ref.so, or its recorded answers where that build is
+    absent: tests/reference_replay.py)."""
     rng = np.random.default_rng(5)
-    for _ in range(3000):
-        x0, y0, x1, y1 = (int(v) for v in rng.integers(0, 300, 4))
-        assert np.array_equal(rg.grid_line(x0, y0, x1, y1), port.gmap_grid_line(x0, y0, x1, y1))
+    segs = [tuple(int(v) for v in rng.integers(0, 300, 4)) for _ in range(3000)]
+
+    def cells(grid_line):
+        lines = [grid_line(*q) for q in segs]
+        return np.array([len(c) for c in lines]), np.concatenate(lines)
+    n_ref, cells_ref = reference.call("grid_line x3000", lambda ss: cells(rg.grid_line), segs)
+    n, c = cells(port.gmap_grid_line)
+    assert np.array_equal(n, n_ref) and same(c, cells_ref)
     laser = pkg.synth.Laser()
     ang = (np.float32(laser.min_angle) + np.arange(1081, dtype=np.float32) * np.float32(laser.angular_resolution)).astype(np.float64)
-    a, b = rg.RefGMap(-25, -25, 25, 25, 0.1), port.PortGMap(-25, -25, 25, 25, 0.1)
+    a, b = reference.new(rg.RefGMap, -25, -25, 25, 25, 0.1), port.PortGMap(-25, -25, 25, 25, 0.1)
     for seed in range(4):  # several scans accumulated into one map
         r = pkg.synth.make_match_case(50 + seed).ranges.astype(np.float32).astype(np.float64)
         assert a.compute_map(r, ang, (0.2 * seed, -0.1 * seed)) == 0
         assert b.compute_map(r, ang, (0.2 * seed, -0.1 * seed)) == 0
     for x, y in zip(a.cells()[:4], b.cells()):
-        assert np.array_equal(x, y)
-    occ = a.cells()[4]
+        assert same(y, x)
+    unknown, occupied = reference.call("occupancy classes", lambda: (a.cells()[4] < 0, a.cells()[4] > 0.25))
     ros = b.ros_map()[:b.size_y, :b.size_x]  # the 500x500 published map holds the 480x480 patch-rounded storage
-    assert ((ros == -1) == (occ < 0)).all() and ((ros == 100) == (occ > 0.25)).all()
+    assert same(ros == -1, unknown) and same(ros == 100, occupied)
     # a ray leaving the map: the reference would assert; both report an error and change nothing
-    c, d = rg.RefGMap(-5, -5, 5, 5, 0.05), port.PortGMap(-5, -5, 5, 5, 0.05)
+    c, d = reference.new(rg.RefGMap, -5, -5, 5, 5, 0.05), port.PortGMap(-5, -5, 5, 5, 0.05)
     assert c.compute_map(np.full(1081, 20.0), ang) == -1 and d.compute_map(np.full(1081, 20.0), ang) == -1
     assert d.visits.sum() == 0
     a.close(); c.close()

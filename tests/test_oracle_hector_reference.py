@@ -1,6 +1,6 @@
 """CPU tests pinning the Hector restatement (oracle/hector_oracle.c) to the reference: the UNMODIFIED lesson4 headers
-compiled against the Eigen stand-in (oracle/ref_hector.cpp -> oracle/_ref/libhector_ref.so, live where it was built)
-and the golden vectors that build produced (tests/golden/hector.npz, always).  Integers (update indices, Bresenham
+compiled against the Eigen stand-in (oracle/ref_hector.cpp -> oracle/_ref/libhector_ref.so where it was built, its
+recorded answers elsewhere: tests/reference_replay.py) and the golden vectors that build produced (tests/golden/hector.npz).  Integers (update indices, Bresenham
 cells) and float32 log-odds / poses / Hessians are compared bit for bit."""
 import os
 
@@ -8,9 +8,9 @@ import numpy as np
 import pytest
 
 from oracle import port, ref_hector as rh
+from reference_replay import same_bits
 
 G = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
-live = pytest.mark.skipif(not rh.available(), reason="oracle/_ref/libhector_ref.so not built")
 
 
 def data_container(laser, ranges, res=0.05, max_dist=20.0, min_dist=0.4):
@@ -28,16 +28,15 @@ def data_container(laser, ranges, res=0.05, max_dist=20.0, min_dist=0.4):
 
 def same_maps(a, b):
     (la, ua), (lb, ub) = a, b
-    return np.array_equal(ua, ub) and np.array_equal(la.view(np.int32), lb.view(np.int32))
+    return same_bits(ua, ub) and same_bits(la, lb)
 
 
-@live
-def test_update_by_scan_bit_exact(pkg):
+def test_update_by_scan_bit_exact(pkg, reference):
     laser = pkg.synth.Laser()
     for seed in range(6):
         mc = pkg.synth.make_match_case(100 + seed, dropout=0.02)
         pts = data_container(laser, mc.base_ranges)
-        a, b = port.PortHectorMap(1024, 1024, 0.05), rh.RefHectorMap(1024, 1024, 0.05)
+        a, b = port.PortHectorMap(1024, 1024, 0.05), reference.new(rh.RefHectorMap, 1024, 1024, 0.05)
         a.set_factors(0.4, 0.9), b.set_factors(0.4, 0.9)
         for k in range(4):  # moving pose, sub-cell origo offsets
             pose = mc.base_pose.astype(np.float32) + np.float32(0.013 * k)
@@ -50,41 +49,38 @@ def test_update_by_scan_bit_exact(pkg):
         a.close(), b.close()
 
 
-@live
-def test_update_random_clouds_and_map_edges():
+def test_update_random_clouds_and_map_edges(reference):
     """Beams that start or end outside the map are dropped whole (OccGridMapBase.h:236-247); tiny maps, both axes."""
     rng = np.random.default_rng(3)
     for sx, sy, res in ((64, 64, 0.1), (200, 120, 0.05), (33, 257, 0.2)):
-        a, b = port.PortHectorMap(sx, sy, res), rh.RefHectorMap(sx, sy, res)
+        a, b = port.PortHectorMap(sx, sy, res), reference.new(rh.RefHectorMap, sx, sy, res)
         for k in range(5):
             pts = rng.uniform(-1.2 * max(sx, sy), 1.2 * max(sx, sy), (400, 2)).astype(np.float32)
             pose = np.array([rng.uniform(-1, 1) * sx * res * 0.4, rng.uniform(-1, 1) * sy * res * 0.4,
                              rng.uniform(-np.pi, np.pi)], np.float32)
             o = rng.uniform(-3, 3, 2).astype(np.float32)
             a.update_by_scan(pts, o, pose), b.update_by_scan(pts, o, pose)
-        assert same_maps(a.cells(), b.cells()) and (b.cells()[1] >= 0).sum() > 100
+        assert same_maps(a.cells(), b.cells()) and (a.cells()[1] >= 0).sum() > 100
         a.close(), b.close()
 
 
-@live
-def test_update_by_scan_just_once_bit_exact():
+def test_update_by_scan_just_once_bit_exact(reference):
     rng = np.random.default_rng(9)
-    a, b = port.PortHectorMap(1601, 1601, 0.05), rh.RefHectorMap(1601, 1601, 0.05)
+    a, b = port.PortHectorMap(1601, 1601, 0.05), reference.new(rh.RefHectorMap, 1601, 1601, 0.05)
     for _ in range(3):
         p = rng.uniform(-25, 25, (700, 2)).astype(np.float32)
         a.update_by_scan_just_once(p, (0, 0)), b.update_by_scan_just_once(p, (0, 0))
     assert same_maps(a.cells(), b.cells())
 
 
-@live
-def test_match_data_bit_exact(pkg):
+def test_match_data_bit_exact(pkg, reference):
     laser = pkg.synth.Laser()
     converged = 0
     for seed in range(25):
         mc = pkg.synth.make_match_case(200 + seed)
         pts = data_container(laser, mc.base_ranges)
         pose = mc.base_pose.astype(np.float32)
-        a, b = port.PortHectorMap(1024, 1024, 0.05), rh.RefHectorMap(1024, 1024, 0.05)
+        a, b = port.PortHectorMap(1024, 1024, 0.05), reference.new(rh.RefHectorMap, 1024, 1024, 0.05)
         a.set_factors(0.4, 0.9), b.set_factors(0.4, 0.9)
         for _ in range(3):
             a.update_by_scan(pts, (0, 0), pose), b.update_by_scan(pts, (0, 0), pose)
@@ -108,41 +104,43 @@ def run_stream(proc, laser, ranges, start_pose, first_without_matching):
     return np.array(out, np.float32)
 
 
-@live
 @pytest.mark.parametrize("first_without_matching", [False, True])
-def test_processor_stream_bit_exact(pkg, first_without_matching):
+def test_processor_stream_bit_exact(pkg, reference, first_without_matching):
     """HectorSlamProcessor::update over a 3-level MapRepMultiMap on a 60-scan trajectory: every pose, every Hessian
     and all three final maps equal the reference's bit for bit."""
     laser = pkg.synth.Laser()
     _, poses, ranges = pkg.synth.make_trajectory(31, 60, laser, step_xy=0.12, step_th_deg=2.0)
     kw = dict(resolution=0.05, size_x=1000, size_y=1000, start=(0.5, 0.5), levels=3, min_dist=0.15, min_angle=0.06)
-    a, b = port.PortHectorProcessor(**kw), rh.RefHectorProcessor(**kw)
+    a, b = port.PortHectorProcessor(**kw), reference.new(rh.RefHectorProcessor, **kw)
     ta = run_stream(a, laser, ranges, poses[0], first_without_matching)
     tb = run_stream(b, laser, ranges, poses[0], first_without_matching)
     assert np.array_equal(ta.view(np.int32), tb.view(np.int32))
     n_updates = []
     for lvl in range(3):
         assert same_maps(a.level(lvl), b.level(lvl))
-        n_updates.append((b.level(lvl)[1].max() + 1) // 3)
+        n_updates.append((a.level(lvl)[1].max() + 1) // 3)
     assert n_updates[0] >= 4 and n_updates[0] == n_updates[1] == n_updates[2]
     assert np.abs(tb[-1, :2] - poses[-1, :2]).max() < 0.05
     a.close(), b.close()
 
 
-@live
-def test_processor_angle_gate_truncates(pkg):
+def test_processor_angle_gate_truncates(pkg, reference):
     """UtilFunctions.h:88 calls the unqualified abs() with only <cmath> included -> int abs(int): a 0.5 rad turn does
     NOT trigger a map update with angleDiffThresh 0.13, a 1.2 rad turn does.  Restatement and reference agree."""
     laser = pkg.synth.Laser()
     mc = pkg.synth.make_match_case(7)
     pts = data_container(laser, mc.base_ranges)
+
+    def map_updates(proc, pts, turn):
+        proc.update(pts, (0, 0), np.zeros(3, np.float32), True)
+        proc.update(pts, (0, 0), np.array([0, 0, turn], np.float32), False)
+        n = (proc.level(0)[1].max() + 1) // 3
+        proc.close()
+        return n
     for turn, expect in ((0.5, 1), (1.2, 2)):
-        n = []
-        for proc in (port.PortHectorProcessor(size_x=512, size_y=512), rh.RefHectorProcessor(size_x=512, size_y=512)):
-            proc.update(pts, (0, 0), np.zeros(3, np.float32), True)
-            proc.update(pts, (0, 0), np.array([0, 0, turn], np.float32), False)
-            n.append((proc.level(0)[1].max() + 1) // 3)
-            proc.close()
+        n = [map_updates(port.PortHectorProcessor(size_x=512, size_y=512), pts, turn),
+             reference.call("map updates after a turn",
+                            lambda p, t: map_updates(rh.RefHectorProcessor(size_x=512, size_y=512), p, t), pts, turn)]
         assert n == [expect, expect], (turn, n)
 
 
@@ -172,8 +170,7 @@ def test_hector_golden(pkg):
     assert np.array_equal(lo.ravel()[idx].view(np.int32), g["jo_lo"].view(np.int32))
 
 
-@live
-def test_grid_probability_double_exp(pkg):
+def test_grid_probability_double_exp(pkg, reference):
     """getGridProbability (GridMapLogOdds.h:136-140): the unqualified exp() on a float is the C library's double exp,
     rounded to float (the reference build imports `exp`, not `expf`).  2^20 log-odds values incl. every multiple-sum
     the update factors can produce: restatement == reference, bit for bit; and the expf reading would NOT be."""
@@ -182,12 +179,15 @@ def test_grid_probability_double_exp(pkg):
     lf, lo_ = np.float32(np.log(np.float32(0.4) / np.float32(0.6))), np.float32(np.log(np.float32(0.9) / np.float32(0.1)))
     combos = (np.arange(-60, 1, dtype=np.float32)[:, None] * lf + np.arange(0, 40, dtype=np.float32)[None, :] * lo_).ravel()
     v = np.concatenate([combos, rng.uniform(-60, 60, (1 << 20) - len(combos)).astype(np.float32)]).astype(np.float32)
-    a, b = np.zeros_like(v), np.zeros_like(v)
-    L = port.lib()
-    L.orc_hector_grid_probabilities(v.ctypes.data_as(C.POINTER(C.c_float)), len(v), a.ctypes.data_as(C.POINTER(C.c_float)))
-    rh.lib().ref_hector_grid_probabilities(v.ctypes.data_as(C.POINTER(C.c_float)), len(v), b.ctypes.data_as(C.POINTER(C.c_float)))
-    assert np.array_equal(a.view(np.int32), b.view(np.int32))
+
+    def probabilities(fn, v):
+        out = np.zeros_like(v)
+        fn(v.ctypes.data_as(C.POINTER(C.c_float)), len(v), out.ctypes.data_as(C.POINTER(C.c_float)))
+        return out
+    a = probabilities(port.lib().orc_hector_grid_probabilities, v)
+    b = reference.call("grid probabilities", lambda x: probabilities(rh.lib().ref_hector_grid_probabilities, x), v)
+    assert same_bits(a, b)
     with np.errstate(all="ignore"):
         odds_f = np.exp(v)  # numpy float32 exp: the other reading
         alt = odds_f / (odds_f + np.float32(1.0))
-    assert (alt.view(np.int32) != b.view(np.int32)).any()
+    assert (alt.view(np.int32) != a.view(np.int32)).any()  # a is b, bit for bit
