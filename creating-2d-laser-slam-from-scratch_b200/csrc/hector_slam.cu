@@ -30,7 +30,6 @@
 #include <algorithm>
 #include <atomic>
 #include <cmath>
-#include <cstdlib>
 #include <cstring>
 #include <new>
 #include <vector>
@@ -80,9 +79,6 @@ struct HsState {  // device-resident state of ONE processor
   int bb_x0[HS_L], bb_y0[HS_L], bb_x1[HS_L], bb_y1[HS_L];  // cells the update's rays can touch (inclusive; empty: x1 < x0)
   unsigned long long visits, n_matched, n_updated;
   unsigned long long t_match_ns, t_update_ns;
-  unsigned long long hfine[8]; // warp 0 of helper CTA 1 (cluster match): [0] waiting for the pose, [1..5] as fine[0..4], [6] column sum, [7] iterations
-  unsigned long long fine[8];  // thread 0's view of the per-point phase: [0] pose read + transform, [1] cell load to use, [2] term arithmetic, [3] warp reduction + store, [4] barrier
-  unsigned long long prof[8];  // SM cycles of processor 0's matching CTA: [0] staging, [1] point terms, [2] sums, [3] solve, [4] trig, [5] gate + bbox, [6] iterations
 };
 
 struct HsBatch {  // kernel parameter
@@ -90,8 +86,6 @@ struct HsBatch {  // kernel parameter
   int levels, batch, cap;
   float lo_free, lo_occ, min_dist, min_angle;
   int exact, use_fma;
-  int l2_loads;    // 1: the match reads the probability planes with ld.global.cg (tuning switch B2S_HS_L2_LOADS)
-  int master_share;  // cluster match: 1 = the solving CTA also takes a share of the points, 0 = only the helpers do
   HsState *state;  // [batch]
 };
 
@@ -184,7 +178,7 @@ struct HsFetch {
   float i0, i1, i2, i3, fx, fy;
   bool inside;
 };
-__device__ __forceinline__ HsFetch hs_fetch(const float4 *__restrict__ quad, int sx, int sy, float x, float y, bool l2) {
+__device__ __forceinline__ HsFetch hs_fetch(const float4 *__restrict__ quad, int sx, int sy, float x, float y) {
   HsFetch f;
   const float lim_x = (float)sx - 2.0f, lim_y = (float)sy - 2.0f;  // setMapCellDims: dims - 2
   f.inside = !(x < 0.0f || x > lim_x || y < 0.0f || y > lim_y);
@@ -193,7 +187,7 @@ __device__ __forceinline__ HsFetch hs_fetch(const float4 *__restrict__ quad, int
     const int ix = (int)x, iy = (int)y;
     f.fx = x - (float)ix; f.fy = y - (float)iy;
     const float4 *c = quad + (iy * sx + ix);
-    const float4 q = l2 ? __ldcg(c) : *c;
+    const float4 q = *c;
     f.i0 = q.x; f.i1 = q.y; f.i2 = q.z; f.i3 = q.w;
   }
   return f;
@@ -238,9 +232,9 @@ __device__ inline bool hs_pose_difference_larger_than(const float a[3], const fl
 
 // terms of one point for getCompleteHessianDerivs (OccGridMapUtil.h:99-126)
 __device__ __forceinline__ HsFetch hs_point_fetch(const float4 *__restrict__ prob, int sx, int sy, float2 p, float c, float s,
-                                                  float e0, float e1, bool l2) {
+                                                  float e0, float e1) {
   const float tx = (c * p.x + (-s) * p.y) + e0, ty = (s * p.x + c * p.y) + e1;
-  return hs_fetch(prob, sx, sy, tx, ty, l2);
+  return hs_fetch(prob, sx, sy, tx, ty);
 }
 __device__ __forceinline__ void hs_point_terms(const HsFetch &f, float2 p, float sin_rot, float cos_rot, float a[9]) {
   float t[3];
@@ -328,37 +322,21 @@ __device__ __forceinline__ HsLine hs_line(float c, float s, float mx, float my, 
 // form), so: only the warps that own points run it, every thread stores its nine terms as columns (9 STS instead of a
 // 45-shuffle tree per warp), and warps 0..8 then sum one column each.  Returns sum `warp` in every lane of warps 0..8.
 // Contains one __syncthreads.
-struct HsTicks {  // thread 0's cycle stamps (clock reads pinned behind a value by the asm's unused input)
-  unsigned long long fine[8];
-  long long mark;
-  __device__ __forceinline__ void tick(int slot, float dep) {
-    long long c_;
-    asm volatile("mov.u64 %0, %%clock64;" : "=l"(c_) : "f"(dep) : "memory");
-    if (slot >= 0) fine[slot] += (unsigned long long)(c_ - mark);
-    mark = c_;
-  }
-};
 __device__ __forceinline__ float hs_share_sums(const float4 *__restrict__ prob, int sx, int sy, const float2 *pts, int cnt,
                                                float factor, float e0, float e1, float c, float s, float sin_rot,
-                                               float cos_rot, bool l2, float *terms, int pitch, int tid, int lane, int warp,
-                                               HsTicks *tk = nullptr) {
-  if (tk && warp == 0) tk->tick(5, e0);  // since the end of the previous solve: publish + barrier + loop head
+                                               float cos_rot, float *terms, int pitch, int tid, int lane, int warp) {
   if (warp * 32 < cnt) {
 #pragma unroll 1
     for (int i = tid; i < cnt; i += HS_THREADS) {
       const float2 p = make_float2(__fmul_rn(pts[i].x, factor), __fmul_rn(pts[i].y, factor));
-      const HsFetch f = hs_point_fetch(prob, sx, sy, p, c, s, e0, e1, l2);
-      if (tk && warp == 0) { tk->tick(0, f.fx); tk->tick(1, f.i0); }
+      const HsFetch f = hs_point_fetch(prob, sx, sy, p, c, s, e0, e1);
       float t[9];
       hs_point_terms(f, p, sin_rot, cos_rot, t);
-      if (tk && warp == 0) tk->tick(2, t[2] + t[5]);
 #pragma unroll
       for (int q = 0; q < 9; q++) terms[q * pitch + i] = t[q];
     }
   }
-  if (tk && warp == 0) tk->tick(3, e0);
   __syncthreads();
-  if (tk && warp == 0) tk->tick(4, e0);
   float v = 0.0f;
   if (warp < 9) {
     const float *col = terms + warp * pitch;
@@ -374,7 +352,6 @@ __device__ __forceinline__ float hs_share_sums(const float4 *__restrict__ prob, 
 #pragma unroll
     for (int d = 16; d > 0; d >>= 1) v += __shfl_xor_sync(0xffffffffu, v, d);
   }
-  if (tk && warp == 0) tk->tick(6, v);
   return v;
 }
 
@@ -385,18 +362,17 @@ __host__ __device__ inline size_t hs_smem_bytes(int cap) { return hs_terms_offse
 
 // MapRepMultiMap::matchData (:144-166) on every level, coarsest first, + the gate and the update parameters of
 // HectorSlamProcessor::update (:81-108), by ONE CTA for processor b.
-// Returns the gate's verdict (map update or not).  `s_prof`: [16] shared-memory profile counters of the calling kernel
-// (flushed to the state once per launch: sixteen global read-modify-writes per scan were ~0.4 us of the serial tail).
+// Returns the gate's verdict (map update or not).
 template <bool EXACT, bool CLUSTER>
-__device__ bool hs_match_cta(const HsBatch &P, const HsCall &C, int b, unsigned char *smem, unsigned long long *s_prof,
-                             HsXchg *xc = nullptr, uint32_t *xc_parity = nullptr) {
+__device__ bool hs_match_cta(const HsBatch &P, const HsCall &C, int b, unsigned char *smem, HsXchg *xc = nullptr,
+                             uint32_t *xc_parity = nullptr) {
   static_assert(!(EXACT && CLUSTER), "the bit-exact sums are one sequential chain: nothing to split");
   HsState *st = P.state + b;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   constexpr int NW = HS_THREADS / 32;
   const int n = C.n0 ? C.n0[b] : C.n0_uniform;
   constexpr bool exact = EXACT;  // compile-time: each mode's kernel carries only its own code
-  const bool use_fma = P.use_fma != 0, l2 = P.l2_loads != 0;
+  const bool use_fma = P.use_fma != 0;
   float2 *spts = reinterpret_cast<float2 *>(smem);
   float *terms = reinterpret_cast<float *>(smem + hs_terms_offset(P.cap));
   const int pitch = hs_pitch(P.cap);
@@ -409,10 +385,7 @@ __device__ bool hs_match_cta(const HsBatch &P, const HsCall &C, int b, unsigned 
   const uint32_t csize = CLUSTER ? hs_cluster_size() : 1u;
   uint32_t part_parity = CLUSTER ? *xc_parity : 0u;
   int my0 = 0, my1 = n;  // this CTA's share of the points in the per-point phase
-  if (CLUSTER) {
-    if (P.master_share || csize < 2) hs_share(n, 0, (int)csize, my0, my1);
-    else my1 = 0;  // the helpers cover the whole scan; this CTA only solves
-  }
+  if (CLUSTER) hs_share(n, 0, (int)csize, my0, my1);
   if (CLUSTER && tid == 0) s_lost = 0;
   // master -> helpers: the pose of the next iteration (bc[0..6]) into every helper's HsXchg::pose; one st.async per lane
   // of warp 0 (the solving thread publishes nothing itself: 21 serial remote stores cost it ~300 cycles)
@@ -437,15 +410,6 @@ __device__ bool hs_match_cta(const HsBatch &P, const HsCall &C, int b, unsigned 
     for (int q = 0; q < 9; q++) lcov[q] = st->last_cov[q];
   }
   const unsigned long long t0 = hs_now_ns();
-  long long c_mark = clock64();
-  unsigned long long pf[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-#define HS_PROF(slot) do { if (tid == 0) { const long long c_now = clock64(); pf[slot] += (unsigned long long)(c_now - c_mark); c_mark = c_now; } } while (0)
-  // clock reads pinned behind a value (the asm's unused input), so that they bracket the instruction that produces it
-  HsTicks tk;
-#pragma unroll
-  for (int q = 0; q < 8; q++) tk.fine[q] = 0;
-  tk.mark = clock64();
-#define HS_TICK(slot, dep) do { if (tid == 0) tk.tick((slot), (dep)); } while (0)
   const float2 *gp = reinterpret_cast<const float2 *>(C.pts0) + (size_t)b * C.pts_stride;
   for (int i = tid; i < n; i += HS_THREADS) {
     const float2 p = gp[i];
@@ -457,7 +421,6 @@ __device__ bool hs_match_cta(const HsBatch &P, const HsCall &C, int b, unsigned 
     s_world[0] = h[0]; s_world[1] = h[1]; s_world[2] = h[2];
   }
   __syncthreads();
-  HS_PROF(0);
   float world0 = s_world[0], world1 = s_world[1], world2 = s_world[2];
   bool any = false;
   if (!C.map_without_matching && n > 0) {
@@ -485,8 +448,7 @@ __device__ bool hs_match_cta(const HsBatch &P, const HsCall &C, int b, unsigned 
         const float e0 = bc[0], e1 = bc[1], c = bc[3], s = bc[4], sin_rot = bc[5], cos_rot = bc[6];
         if constexpr (CLUSTER) {
           float v = 0.0f;
-          if (my1 > 0) v = hs_share_sums(prob, m.sx, m.sy, spts, my1, factor, e0, e1, c, s, sin_rot, cos_rot, l2, terms, pitch, tid, lane, warp);
-          HS_PROF(1);
+          if (my1 > 0) v = hs_share_sums(prob, m.sx, m.sy, spts, my1, factor, e0, e1, c, s, sin_rot, cos_rot, terms, pitch, tid, lane, warp);
           if (warp < 9) {
             if (csize > 1) {  // + the helpers' partial sums, in rank order
               if (tid == 0) hs_mbar_expect_tx(&xc->bar_part, 36u * (csize - 1));
@@ -502,18 +464,15 @@ __device__ bool hs_match_cta(const HsBatch &P, const HsCall &C, int b, unsigned 
         float acc[9];
 #pragma unroll
         for (int q = 0; q < 9; q++) acc[q] = 0.0f;
-        HS_TICK(-1, e0);
         for (int base = my0; base < my1; base += 2 * HS_THREADS) {  // two points per thread, their eight cell loads in flight together
           const int ia = base + tid, ib = base + tid + HS_THREADS;
           const int n = my1;  // (shadows the scan length inside the per-point phase: this CTA's share ends at my1)
           float2 pa = make_float2(0.0f, 0.0f), pb = pa;
           HsFetch fa, fb;
           fa.inside = fb.inside = false;
-          if (ia < n) { pa = make_float2(__fmul_rn(spts[ia].x, factor), __fmul_rn(spts[ia].y, factor)); fa = hs_point_fetch(prob, m.sx, m.sy, pa, c, s, e0, e1, l2); }
-          if (ib < n) { pb = make_float2(__fmul_rn(spts[ib].x, factor), __fmul_rn(spts[ib].y, factor)); fb = hs_point_fetch(prob, m.sx, m.sy, pb, c, s, e0, e1, l2); }
+          if (ia < n) { pa = make_float2(__fmul_rn(spts[ia].x, factor), __fmul_rn(spts[ia].y, factor)); fa = hs_point_fetch(prob, m.sx, m.sy, pa, c, s, e0, e1); }
+          if (ib < n) { pb = make_float2(__fmul_rn(spts[ib].x, factor), __fmul_rn(spts[ib].y, factor)); fb = hs_point_fetch(prob, m.sx, m.sy, pb, c, s, e0, e1); }
           float ta[9], tb[9];
-          HS_TICK(0, fa.fx);
-          HS_TICK(1, fa.i0);
           if (ia < n) {
             hs_point_terms(fa, pa, sin_rot, cos_rot, ta);
             if (exact) {
@@ -535,7 +494,6 @@ __device__ bool hs_match_cta(const HsBatch &P, const HsCall &C, int b, unsigned 
             }
           }
         }
-        HS_TICK(2, acc[8]);
         if (!exact) {
 #pragma unroll
           for (int q = 0; q < 9; q++) {
@@ -547,10 +505,7 @@ __device__ bool hs_match_cta(const HsBatch &P, const HsCall &C, int b, unsigned 
             for (int q = 0; q < 9; q++) terms[q * NW + warp] = acc[q];
           }
         }
-        HS_TICK(3, acc[8]);
         __syncthreads();
-        HS_TICK(4, acc[0]);
-        HS_PROF(1);
         if (exact) {
           // The reference's float32 sums, in point order (OccGridMapUtil.h:99-126): ONE warp instruction advances all nine
           // chains (lane q owns sum q), so the floor is one dependent FADD per point.  (Nine warps with one chain each
@@ -585,7 +540,6 @@ __device__ bool hs_match_cta(const HsBatch &P, const HsCall &C, int b, unsigned 
           __syncwarp();
         }
         }  // !CLUSTER
-        HS_PROF(2);
         if (tid == 0) {  // estimateTransformationLogLh (ScanMatcher.h:107-141)
           const float dTr[3] = {tot[0], tot[1], tot[2]};
           float Hm[9];
@@ -600,14 +554,10 @@ __device__ bool hs_match_cta(const HsBatch &P, const HsCall &C, int b, unsigned 
             n0 += dir[0]; n1 += dir[1]; n2 += dir[2];
           }
           bc[0] = n0; bc[1] = n1; bc[2] = n2;
-          HS_PROF(3);
           if (it + 1 < m.iterations) {
             const HsTrig tr = hs_trig(n2, exact, use_fma);
             bc[3] = tr.c; bc[4] = tr.s; bc[5] = tr.sin_rot; bc[6] = tr.cos_rot;
           }
-          HS_PROF(4);
-          tk.tick(-1, n2);
-          pf[6] += 1;
         }
         if (CLUSTER && warp == 0 && it + 1 < m.iterations) {
           __syncwarp();
@@ -725,14 +675,7 @@ __device__ bool hs_match_cta(const HsBatch &P, const HsCall &C, int b, unsigned 
       st->bb_x1[tid] = s_bb[tid][2]; st->bb_y1[tid] = s_bb[tid][3];  // no ray: max < min -> an empty box
     }
   }
-  HS_PROF(5);
-  if (tid == 0) {
-    if (b == 0) {
-#pragma unroll
-      for (int q = 0; q < 8; q++) { s_prof[q] += pf[q]; s_prof[8 + q] += tk.fine[q]; }
-    }
-    st->t_match_ns = hs_now_ns() - t0;
-  }
+  if (tid == 0) st->t_match_ns = hs_now_ns() - t0;
   if (CLUSTER) *xc_parity = part_parity;
   const bool verdict = s_do != 0;
   if (C.tag) {
@@ -741,12 +684,6 @@ __device__ bool hs_match_cta(const HsBatch &P, const HsCall &C, int b, unsigned 
       asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(C.out + 16 * (size_t)b + 15), "r"(C.tag) : "memory");
   }
   return verdict;
-#undef HS_PROF
-#undef HS_TICK
-}
-
-__device__ __forceinline__ void hs_prof_flush(HsState *st, const unsigned long long *s_prof) {
-  for (int q = 0; q < 8; q++) { st->prof[q] += s_prof[q]; st->fine[q] += s_prof[8 + q]; }
 }
 
 // every CTA but the matching one: wait until scan i's row carries this launch's tag, then read the gate's verdict
@@ -773,22 +710,15 @@ __device__ void hs_match_helper(const HsBatch &P, const HsCall &C, unsigned char
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int n = C.n0_uniform;
   if (C.map_without_matching || n <= 0) return;
-  const bool l2 = P.l2_loads != 0;
   float2 *spts = reinterpret_cast<float2 *>(smem);
   float *terms = reinterpret_cast<float *>(smem + hs_terms_offset(P.cap));
   int p0, p1;
-  if (P.master_share) hs_share(n, (int)rank, (int)csize, p0, p1);
-  else hs_share(n, (int)rank - 1, (int)csize - 1, p0, p1);
+  hs_share(n, (int)rank, (int)csize, p0, p1);
   const int cnt = p1 - p0;
   const float2 *gp = reinterpret_cast<const float2 *>(C.pts0);
   for (int i = tid; i < cnt; i += HS_THREADS) spts[i] = gp[p0 + i];
   __syncthreads();
   const int pitch = hs_pitch(P.cap);
-  HsTicks htk;
-#pragma unroll
-  for (int q = 0; q < 8; q++) htk.fine[q] = 0;
-  htk.mark = clock64();
-  int n_it = 0;
   const uint32_t r_part = hs_mapa(hs_smem_u32(&xc->part[rank][0]), 0), r_bar = hs_mapa(hs_smem_u32(&xc->bar_part), 0);
   float factor = 1.0f;
   for (int l = 1; l < P.levels; l++) factor *= 0.5f;
@@ -803,19 +733,10 @@ __device__ void hs_match_helper(const HsBatch &P, const HsCall &C, unsigned char
       // which are sent after the column reads — but that chain runs through another CTA, which compute-sanitizer's
       // racecheck cannot follow: the barrier (~50 cycles) keeps the tool's report clean.
       __syncthreads();
-      if (warp == 0) { htk.tick(7, xc->pose[0]); n_it++; }
       const float e0 = xc->pose[0], e1 = xc->pose[1], c = xc->pose[3], s = xc->pose[4], sin_rot = xc->pose[5], cos_rot = xc->pose[6];
-      const float v = hs_share_sums(prob, m.sx, m.sy, spts, cnt, factor, e0, e1, c, s, sin_rot, cos_rot, l2, terms, pitch, tid, lane, warp, &htk);
+      const float v = hs_share_sums(prob, m.sx, m.sy, spts, cnt, factor, e0, e1, c, s, sin_rot, cos_rot, terms, pitch, tid, lane, warp);
       if (warp < 9 && lane == 0) hs_st_async(r_part + 4 * warp, v, r_bar);
-      if (warp == 0) htk.tick(-1, v);
     }
-  }
-  if (rank == 1 && tid == 0) {  // the helper's view of an iteration, for b2s_hector_slam_profile_fine
-    HsState *st = P.state;
-    st->hfine[0] += htk.fine[7];
-    for (int q = 0; q < 5; q++) st->hfine[1 + q] += htk.fine[q];
-    st->hfine[6] += htk.fine[6];
-    st->hfine[7] += (unsigned long long)n_it;
   }
 }
 
@@ -959,14 +880,12 @@ __device__ void hs_apply_pass(const HsBatch &P, int b, int w, int nw, int lane) 
 }
 
 // ---- batch path: three launches per step over all B processors ----
+// The matching kernels ask for one CTA per SM: the Gauss-Newton loop keeps its terms in registers (90-96 per thread).
+// Without the minimum ptxas may cap them at 56 so that two CTAs fit, and spill inside the per-point phase.
 template <bool EXACT>
-__global__ void __launch_bounds__(HS_THREADS) k_hs_match(HsBatch P, HsCall C) {
+__global__ void __launch_bounds__(HS_THREADS, 1) k_hs_match(HsBatch P, HsCall C) {
   extern __shared__ __align__(16) unsigned char hs_smem[];
-  __shared__ unsigned long long s_prof[16];
-  if (threadIdx.x < 16) s_prof[threadIdx.x] = 0;
-  __syncthreads();
-  hs_match_cta<EXACT, false>(P, C, blockIdx.x, hs_smem, s_prof);
-  if (blockIdx.x == 0 && threadIdx.x == 0) hs_prof_flush(P.state, s_prof);
+  hs_match_cta<EXACT, false>(P, C, blockIdx.x, hs_smem);
 }
 __global__ void __launch_bounds__(256) k_hs_mark(HsBatch P) {
   const int b = blockIdx.y;
@@ -1018,13 +937,10 @@ struct HsStream {
 };
 
 template <bool EXACT, bool CLUSTER>
-__global__ void __launch_bounds__(HS_THREADS) k_hs_stream(HsBatch P, HsStream S) {
+__global__ void __launch_bounds__(HS_THREADS, 1) k_hs_stream(HsBatch P, HsStream S) {
   extern __shared__ __align__(16) unsigned char hs_smem[];
   __shared__ HsXchg xc;  // same offset in every CTA of the kernel: mapa() of a local address names the peer's copy
-  __shared__ unsigned long long s_prof[16];
   __shared__ int s_flag;
-  if (threadIdx.x < 16) s_prof[threadIdx.x] = 0;
-  __syncthreads();
   uint32_t crank = 0, csize = 1, pose_parity = 0, part_parity = 0;
   if (CLUSTER) {
     crank = hs_cluster_rank();
@@ -1067,7 +983,7 @@ __global__ void __launch_bounds__(HS_THREADS) k_hs_stream(HsBatch P, HsStream S)
     // goes on to the next scan; the other CTAs follow the verdicts and meet it at the update's barriers.  (A grid barrier
     // per scan cost the matching CTA ~1 us: two fences and an L2 round trip.)
     if (blockIdx.x == 0) {
-      update = hs_match_cta<EXACT, CLUSTER>(P, C, 0, hs_smem, s_prof, &xc, &part_parity);
+      update = hs_match_cta<EXACT, CLUSTER>(P, C, 0, hs_smem, &xc, &part_parity);
     } else {
       if (helper) hs_match_helper(P, C, hs_smem, &xc, crank, csize, pose_parity);
       update = hs_wait_decision(C.out, S.tag, &s_flag);
@@ -1082,7 +998,6 @@ __global__ void __launch_bounds__(HS_THREADS) k_hs_stream(HsBatch P, HsStream S)
       if (blockIdx.x == 0 && threadIdx.x == 0) st->t_update_ns = hs_now_ns() - t0;
     }
   }
-  if (blockIdx.x == 0 && threadIdx.x == 0) hs_prof_flush(st, s_prof);
 }
 
 __global__ void k_hs_fill(float *__restrict__ p, size_t n, float v) {
@@ -1103,9 +1018,6 @@ __global__ void k_hs_state_init(HsState *st, int batch, int reset_maps) {
     for (int l = 0; l < HS_L; l++) { s.curr_update_index[l] = 0; s.epoch[l] = 0; s.n_pts[l] = 0; s.origo[l][0] = s.origo[l][1] = 0.0f; }
     s.visits = s.n_matched = s.n_updated = 0;
     s.t_match_ns = s.t_update_ns = 0;
-    for (int q = 0; q < 8; q++) s.prof[q] = 0;
-    for (int q = 0; q < 8; q++) s.fine[q] = 0;
-    for (int q = 0; q < 8; q++) s.hfine[q] = 0;
     for (int l = 0; l < HS_L; l++) { s.bb_x0[l] = s.bb_y0[l] = 0; s.bb_x1[l] = s.bb_y1[l] = -1; }
   }
 }
@@ -1238,8 +1150,6 @@ static b2s_status hs_create(float map_resolution, int map_size_x, int map_size_y
   p->P.lo_occ = hs_prob_to_log_odds(0.6f);
   p->P.min_dist = 0.4f; p->P.min_angle = 0.13f;  // HectorSlamProcessor.h:63-64
   p->P.exact = 1;
-  { const char *e = getenv("B2S_HS_L2_LOADS"); p->P.l2_loads = (e && e[0] == '1') ? 1 : 0; }
-  { const char *e = getenv("B2S_HS_MASTER_SHARE"); p->P.master_share = (e && e[0] == '0') ? 0 : 1; }
   const int variant = glibc_sincosf_variant_of_host();
   p->P.use_fma = variant == 0 ? 0 : 1;
   // MapRepMultiMap ctor (MapRepMultiMap.h:56-89): one offset for every level, dims halve, cell length doubles
@@ -1302,29 +1212,23 @@ static b2s_status hs_create(float map_resolution, int map_size_x, int map_size_y
     HS_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device));
     HS_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_hs_stream<true, false>, HS_THREADS, smem));
     p->coop = coop != 0;
-    int want = HS_STREAM_CTAS;
-    if (const char *ec = getenv("B2S_HS_STREAM_CTAS")) want = std::max(1, atoi(ec));  // tuning switch
-    p->stream_ctas = std::max(1, std::min(want, sms * std::max(per_sm, 0)));
+    p->stream_ctas = std::max(1, std::min(HS_STREAM_CTAS, sms * std::max(per_sm, 0)));
     if (!p->coop) p->stream_ctas = 1;  // without a co-residency guarantee a spinning grid barrier could deadlock
-    // fast mode: the matching CTA's cluster (B2S_HS_CLUSTER=0 switches it off).  Needs the whole cooperative grid
-    // co-resident AS clusters.
-    const char *e = getenv("B2S_HS_CLUSTER");
-    int want_cluster = HS_CLUSTER;
-    if (e && (e[0] == '2' || e[0] == '4' || e[0] == '8')) want_cluster = e[0] - '0';  // tuning switch; 0 switches it off
-    if (p->coop && p->stream_ctas >= want_cluster && !(e && e[0] == '0')) {
+    // fast mode: the matching CTA's cluster.  Needs the whole cooperative grid co-resident AS clusters.
+    if (p->coop && p->stream_ctas >= HS_CLUSTER) {
       cudaLaunchConfig_t cfg;
       std::memset(&cfg, 0, sizeof(cfg));
       cudaLaunchAttribute at[1];
       at[0].id = cudaLaunchAttributeClusterDimension;
-      at[0].val.clusterDim.x = (unsigned)want_cluster; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-      cfg.gridDim = dim3((p->stream_ctas / want_cluster) * want_cluster);
+      at[0].val.clusterDim.x = (unsigned)HS_CLUSTER; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
+      cfg.gridDim = dim3((p->stream_ctas / HS_CLUSTER) * HS_CLUSTER);
       cfg.blockDim = dim3(HS_THREADS);
       cfg.dynamicSmemBytes = smem;
       cfg.attrs = at; cfg.numAttrs = 1;
       int n_clusters = 0;
       if (cudaOccupancyMaxActiveClusters(&n_clusters, k_hs_stream<false, true>, &cfg) == cudaSuccess &&
-          n_clusters * want_cluster >= (int)cfg.gridDim.x)
-        p->cluster = want_cluster;
+          n_clusters * HS_CLUSTER >= (int)cfg.gridDim.x)
+        p->cluster = HS_CLUSTER;
       else
         cudaGetLastError();
     }
@@ -1708,33 +1612,6 @@ b2s_status b2s_hector_slam_stats(b2s_hector_slam *p, double out[5]) {
   for (const HsState &x : s) { out[0] += (double)x.n_matched; out[1] += (double)x.n_updated; out[2] += (double)x.visits; }
   out[3] = (double)s[0].t_match_ns * 1e-6;   // ms of processor 0's last match / update (device %globaltimer)
   out[4] = (double)s[0].t_update_ns * 1e-6;
-  return B2S_OK;
-}
-
-/* SM cycles spent by processor 0's matching CTA since creation, by phase: [0] staging the scan, [1] per-point terms
- * (cell loads + bilinear + products), [2] the nine sums, [3] 3x3 solve, [4] sine / cosine of the new heading,
- * [5] gate + update parameters + ray bounding boxes, [6] Gauss-Newton iterations counted, [7] unused */
-b2s_status b2s_hector_slam_profile(b2s_hector_slam *p, double out[8]) {
-  if (!p || !out) B2S_FAIL(B2S_ERR_BAD_PARAMS, "null argument");
-  B2S_CUDA_CHECK(cudaSetDevice(p->device));
-  HsState s;
-  B2S_CUDA_CHECK(cudaMemcpyAsync(&s, p->d_state, sizeof(HsState), cudaMemcpyDeviceToHost, p->stream));
-  B2S_CUDA_CHECK(cudaStreamSynchronize(p->stream));
-  p->launch_pending = false;
-  for (int q = 0; q < 8; q++) out[q] = (double)s.prof[q];
-  return B2S_OK;
-}
-
-b2s_status b2s_hector_slam_profile_fine(b2s_hector_slam *p, double out[8]) {
-  if (!p || !out) B2S_FAIL(B2S_ERR_BAD_PARAMS, "null argument");
-  B2S_CUDA_CHECK(cudaSetDevice(p->device));
-  HsState s;
-  B2S_CUDA_CHECK(cudaMemcpyAsync(&s, p->d_state, sizeof(HsState), cudaMemcpyDeviceToHost, p->stream));
-  B2S_CUDA_CHECK(cudaStreamSynchronize(p->stream));
-  p->launch_pending = false;
-  for (int q = 0; q < 8; q++) out[q] = (double)s.fine[q];
-  if (p->P.exact == 0 && p->cluster > 1)
-    for (int q = 0; q < 8; q++) out[q] = (double)s.hfine[q];  // the helper's view when the cluster match is in use
   return B2S_OK;
 }
 

@@ -15,10 +15,7 @@
 // All pose arithmetic is double precision in the reference's operation order, so poses, link means and covariances agree
 // with the reference to the matcher's own tolerance (1e-9 in the parity tests) and every threshold decision is the same.
 #include <algorithm>
-#include <chrono>
 #include <cmath>
-#include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <deque>
 #include <list>
@@ -166,14 +163,7 @@ struct CudaBackend {  // the two ScanMatcher instances a Mapper owns, as b2s_mat
   std::vector<double> base_r, base_p;
   std::vector<int32_t> base_rows;
   size_t pool_n[2] = {0, 0};  // scans of the mapper already appended to each handle's device-resident pool
-  double t_pad = 0, t_match = 0, t_create = 0, t_add = 0, t_sweeps = 0;  // seconds, reported at destroy when B2S_MAPPER_PROFILE is set
-  bool profile = std::getenv("B2S_MAPPER_PROFILE") != nullptr;
-  long n_create = 0, n_calls = 0;
   ~CudaBackend() {
-    if (profile)
-      std::fprintf(stderr, "[b2s_mapper] backend: %ld calls, pad-copy %.1f ms, match %.1f ms (upload + rasterise %.1f, sweeps + results %.1f), "
-                           "%ld handle (re)creations %.1f ms\n",
-                   n_calls, 1e3 * t_pad, 1e3 * t_match, 1e3 * t_add, 1e3 * t_sweeps, n_create, 1e3 * t_create);
     for (auto *p : h)
       if (p) b2s_matcher_destroy(p);
   }
@@ -252,10 +242,6 @@ b2s_status cuda_match_ids(b2s_mapper *m, int which, const std::vector<MatchJob> 
                           std::vector<b2s_match_result> &out) {
   CudaBackend *c = m->cuda;
   const int B = (int)jobs.size(), N = m->laser.n_readings;
-  auto now = [] { return std::chrono::steady_clock::now(); };
-  auto secs = [](std::chrono::steady_clock::time_point a, std::chrono::steady_clock::time_point b) { return std::chrono::duration<double>(b - a).count(); };
-  const auto t1 = now();
-  c->n_calls++;
   int max_base = 1;
   for (const MatchJob &j : jobs) {
     if (j.chain.empty()) B2S_FAIL(B2S_ERR_BAD_PARAMS, "mapper: MatchScan against an empty chain");
@@ -282,17 +268,9 @@ b2s_status cuda_match_ids(b2s_mapper *m, int which, const std::vector<MatchJob> 
       c->base_p[3 * k] = sc.corrected.x; c->base_p[3 * k + 1] = sc.corrected.y; c->base_p[3 * k + 2] = sc.corrected.h;
     }
   }
-  const auto t2 = now();
   st = b2s_matcher_set_scans(c->h[which], B, ranges.data(), poses.data());
   if (!st) st = b2s_matcher_add_scans_pool(c->h[which], max_base, c->base_rows.data(), c->base_p.data());
-  if (!st && c->profile) st = b2s_matcher_sync(c->h[which]);
-  const auto t3 = now();
   if (!st) st = b2s_matcher_match_scan(c->h[which], do_penalize ? 1 : 0, do_refine ? 1 : 0, out.data());
-  const auto t4 = now();
-  c->t_pad += secs(t1, t2);
-  c->t_add += secs(t2, t3);
-  c->t_sweeps += secs(t3, t4);
-  c->t_match += secs(t2, t4);
   return st;
 }
 
@@ -335,7 +313,6 @@ b2s_status run_matches(b2s_mapper *m, int which, const std::vector<MatchJob> &jo
 // double on growth so that a stream re-creates it a handful of times at most
 b2s_status cuda_ensure_handle(CudaBackend *c, int which, int batch, int max_base) {
   if (c->h[which] && batch <= c->cap_batch[which] && max_base <= c->cap_base[which]) return B2S_OK;
-  const auto t0 = std::chrono::steady_clock::now();
   if (c->h[which]) b2s_matcher_destroy(c->h[which]);
   c->h[which] = nullptr;
   c->pool_n[which] = 0;
@@ -345,8 +322,6 @@ b2s_status cuda_ensure_handle(CudaBackend *c, int which, int batch, int max_base
   if (st) return st;
   c->cap_batch[which] = cb;
   c->cap_base[which] = cs;
-  c->n_create++;
-  c->t_create += std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
   return B2S_OK;
 }
 
@@ -358,16 +333,12 @@ b2s_status cuda_match(void *user, int which, int batch, const double *ranges, co
                       int do_refine, b2s_match_result *results) {
   CudaBackend *c = static_cast<CudaBackend *>(user);
   const int N = c->laser.n_readings;
-  auto now = [] { return std::chrono::steady_clock::now(); };
-  auto secs = [](std::chrono::steady_clock::time_point a, std::chrono::steady_clock::time_point b) { return std::chrono::duration<double>(b - a).count(); };
-  c->n_calls++;
   int max_base = 1;
   for (int b = 0; b < batch; b++) max_base = std::max(max_base, (int)n_base[b]);
   {
     b2s_status st = cuda_ensure_handle(c, which, batch, max_base);
     if (st) return st;
   }
-  const auto t1 = now();
   for (int b = 0; b < batch; b++)
     if (n_base[b] <= 0) B2S_FAIL(B2S_ERR_BAD_PARAMS, "mapper: MatchScan against an empty chain");
   c->base_r.resize((size_t)batch * max_base * N);
@@ -378,23 +349,8 @@ b2s_status cuda_match(void *user, int which, int batch, const double *ranges, co
       std::memcpy(&c->base_r[dst * N], base_ranges + src * N, sizeof(double) * N);
       std::memcpy(&c->base_p[dst * 3], base_poses + src * 3, sizeof(double) * 3);
     }
-  const auto t2 = now();
-  b2s_status st;
-  if (c->profile) {  // B2S_MAPPER_PROFILE: the three stages separately, with a stream sync after each
-    st = b2s_matcher_set_scans(c->h[which], batch, ranges, poses);
-    if (!st) st = b2s_matcher_add_scans(c->h[which], max_base, c->base_r.data(), c->base_p.data());
-    if (!st) st = b2s_matcher_sync(c->h[which]);
-    const auto t3 = now();
-    if (!st) st = b2s_matcher_match_scan(c->h[which], do_penalize, do_refine, results);
-    c->t_add += secs(t2, t3);
-    c->t_sweeps += secs(t3, now());
-  } else {
-    st = b2s_matcher_match_scan_host(c->h[which], batch, ranges, poses, max_base, c->base_r.data(), c->base_p.data(),
+  return b2s_matcher_match_scan_host(c->h[which], batch, ranges, poses, max_base, c->base_r.data(), c->base_p.data(),
                                      do_penalize, do_refine, results);
-  }
-  c->t_pad += secs(t1, t2);
-  c->t_match += secs(t2, now());
-  return st;
 }
 
 // ---- MapperGraph

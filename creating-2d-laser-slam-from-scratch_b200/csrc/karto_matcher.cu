@@ -26,7 +26,6 @@
 //   k_angular_cov      fine-stage angular covariance (re-evaluates GetResponse at the best cell)
 #include <algorithm>
 #include <cmath>
-#include <cstdlib>
 #include <cstring>
 #include <mutex>
 #include <new>
@@ -879,8 +878,8 @@ struct ReduceArgs {
 };
 
 
-template <int STRIDE, bool GEN, int THREADS>
-__global__ void __launch_bounds__(THREADS, 1)
+template <int STRIDE, bool GEN>
+__global__ void __launch_bounds__(WIN_THREADS, 1)
     k_sweep_window(const uint8_t *__restrict__ grids, size_t grid_pitch, int data_size, int copy_bytes,
                    const int32_t *__restrict__ lists, const int32_t *__restrict__ counts,
                    const int32_t *__restrict__ starts, const int32_t *__restrict__ flags, int batch, int n, int na,
@@ -894,7 +893,7 @@ __global__ void __launch_bounds__(THREADS, 1)
   uint8_t *sgrid = smem;  // [WIN_GUARD zeros][band image][WIN_GUARD zeros]
   __shared__ uint64_t bar;
   __shared__ int s_unit, s_item;
-  __shared__ __align__(16) int32_t s_offsets[THREADS / 32][32];  // per-warp staging of 32 window origins
+  __shared__ __align__(16) int32_t s_offsets[WIN_THREADS / 32][32];  // per-warp staging of 32 window origins
 
   const int lane = threadIdx.x & 31;
   int32_t *s_off = s_offsets[threadIdx.x >> 5];
@@ -2225,7 +2224,7 @@ static b2s_status run_correlate(b2s_matcher *m, const b2s_search *s, bool /*cent
   static size_t win_static = 0;
   if (!win_static) {
     cudaFuncAttributes fa;
-    B2S_CUDA_CHECK(cudaFuncGetAttributes(&fa, k_sweep_window<1, false, WIN_THREADS>));
+    B2S_CUDA_CHECK(cudaFuncGetAttributes(&fa, k_sweep_window<1, false>));
     win_static = fa.sharedSizeBytes;
   }
   const long long smem_limit = (long long)m->smem_optin - (long long)win_static - 512;
@@ -2297,23 +2296,16 @@ static b2s_status run_correlate(b2s_matcher *m, const b2s_search *s, bool /*cent
     // the GEN = false instantiation assumes exactly two lanes per row-start bank (see win_load)
     const int bank_step = ((m->g.width_step >> 2) * std::max(stride, 1)) & 31;
     const bool gen = (bank_step & 3) != 2;
-    // tuning switch: B2S_WIN_THREADS=384 runs the sweep with 12 warps per SM (leaves registers for co-resident kernels)
-    static const int win_threads = [] { const char *e = getenv("B2S_WIN_THREADS"); return (e && atoi(e) == 384) ? 384 : WIN_THREADS; }();
-    auto launch = [&](auto kern, int threads) -> b2s_status {
+    auto launch = [&](auto kern) -> b2s_status {
       B2S_CUDA_CHECK(raise_dyn_smem(kern, win_smem));
-      kern<<<ctas, threads, win_smem, m->stream>>>(m->d_grids, m->grid_pitch, m->g.data_size, copy_bytes, m->d_lists,
+      kern<<<ctas, WIN_THREADS, win_smem, m->stream>>>(m->d_grids, m->grid_pitch, m->g.data_size, copy_bytes, m->d_lists,
                                                    m->d_counts, m->d_starts, m->d_flags, B, n, na, nx, ny,
                                                    m->g.width_step, m->d_sums, m->d_work, band_rows, nbands,
                                                    band_bytes, neg_bands);
       return B2S_OK;
     };
-    if (win_threads == 384) {
-      if (stride == 2) st = gen ? launch(k_sweep_window<2, true, 384>, 384) : launch(k_sweep_window<2, false, 384>, 384);
-      else st = gen ? launch(k_sweep_window<1, true, 384>, 384) : launch(k_sweep_window<1, false, 384>, 384);
-    } else {
-      if (stride == 2) st = gen ? launch(k_sweep_window<2, true, WIN_THREADS>, WIN_THREADS) : launch(k_sweep_window<2, false, WIN_THREADS>, WIN_THREADS);
-      else st = gen ? launch(k_sweep_window<1, true, WIN_THREADS>, WIN_THREADS) : launch(k_sweep_window<1, false, WIN_THREADS>, WIN_THREADS);
-    }
+    if (stride == 2) st = gen ? launch(k_sweep_window<2, true>) : launch(k_sweep_window<2, false>);
+    else st = gen ? launch(k_sweep_window<1, true>) : launch(k_sweep_window<1, false>);
     if (st) return st;
     // matches whose lattice is not the regular raster (a centre exactly on a rounding tie) fall through;
     // they compute their lookup values on the fly (no table was materialised for them)

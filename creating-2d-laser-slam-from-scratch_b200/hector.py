@@ -48,9 +48,7 @@ def _bind():
     L.b2s_hector_slam_copy_level_of.argtypes = [vp, C.c_int, C.c_int, fp, ip]
     L.b2s_hector_slam_last_poses.argtypes = [vp, C.c_int, fp, fp]
     L.b2s_hector_slam_debug_set_epoch.argtypes = [vp, C.c_uint]
-    L.b2s_hector_slam_profile.argtypes = [vp, C.POINTER(C.c_double)]
     L.b2s_hector_slam_match_cluster_size.argtypes = [vp]
-    L.b2s_hector_slam_profile_fine.argtypes = [vp, C.POINTER(C.c_double)]
     _bound = True
     return L
 
@@ -201,19 +199,6 @@ class HectorSlam:
         a, u = np.zeros(3, np.float32), np.zeros(3, np.float32)
         check(self.L.b2s_hector_slam_last_poses(self.h, b, _f(a), _f(u)))
         return a, u
-
-    def profile(self):
-        out = np.zeros(8)
-        check(self.L.b2s_hector_slam_profile(self.h, out.ctypes.data_as(C.POINTER(C.c_double))))
-        it = max(out[6], 1.0)
-        fine = np.zeros(8)
-        check(self.L.b2s_hector_slam_profile_fine(self.h, fine.ctypes.data_as(C.POINTER(C.c_double))))
-        return dict(staging=out[0], terms=out[1], sums=out[2], solve=out[3], trig=out[4], gate=out[5], iterations=out[6],
-                    cycles_per_iteration=dict(terms=out[1] / it, sums=out[2] / it, solve=out[3] / it, trig=out[4] / it),
-                    raw_fine=[float(x) for x in fine],
-                    terms_detail_cycles_per_iteration=dict(transform=fine[0] / it, load_to_use=fine[1] / it,
-                                                           arithmetic=fine[2] / it, reduce=fine[3] / it, barrier=fine[4] / it,
-                                                           loop_head=fine[5] / it, column_sum=fine[6] / it))
 
     def debug_set_epoch(self, updates):
         check(self.L.b2s_hector_slam_debug_set_epoch(self.h, int(updates)))

@@ -454,7 +454,7 @@ b2s_status b2s_hector_slam_stats(b2s_hector_slam *p, double out[5]);
 b2s_status b2s_hector_slam_set_exact(b2s_hector_slam *p, int exact);
 /* Non-exact mode, single-processor handles: the CTAs of one thread-block cluster share the per-point phase of every
  * Gauss-Newton iteration (pose out / nine partial sums back through distributed shared memory).  Returns the CTAs per
- * cluster in use (1: no cluster launch — B2S_HS_CLUSTER=0 or the device cannot co-schedule the grid as clusters). */
+ * cluster in use (1: no cluster launch — the device cannot co-schedule the grid as clusters, or refused the launch). */
 int32_t b2s_hector_slam_match_cluster_size(const b2s_hector_slam *p);
 /* The node's loop over a recorded stream (hector_slam.cc:195-204: update(container, getLastScanMatchPose())) in ONE
  * call: n_scans scans, points concatenated ([sum n_points][2], level-0 map-cell units), hint of scan i = pose of scan
@@ -487,13 +487,6 @@ b2s_status b2s_hector_slam_copy_level_of(b2s_hector_slam *p, int processor, int 
 /* getLastScanMatchPose / getLastMapUpdatePose (HectorSlamProcessor.h:118-119) of one processor; either may be NULL */
 b2s_status b2s_hector_slam_last_poses(b2s_hector_slam *p, int processor, float last_scan_match_pose[3],
                                       float last_map_update_pose[3]);
-/* SM cycles of processor 0's matching CTA since creation, by phase: staging, per-point terms, the nine sums, 3x3 solve,
- * sine / cosine, gate + update parameters, iterations counted, (unused) */
-b2s_status b2s_hector_slam_profile(b2s_hector_slam *p, double out[8]);
-/* the per-point phase as thread 0 of the matching CTA sees it, SM cycles summed over iterations: [0] pose read +
- * point transform, [1] probability-cell load to first use, [2] term arithmetic, [3] warp reduction + store, [4] CTA
- * barrier (waiting for the slowest warp) */
-b2s_status b2s_hector_slam_profile_fine(b2s_hector_slam *p, double out[8]);
 /* test hook: pretend `updates` map updates already consumed per-scan stamp epochs (exercises the 20-bit epoch wrap) */
 b2s_status b2s_hector_slam_debug_set_epoch(b2s_hector_slam *p, unsigned int updates);
 

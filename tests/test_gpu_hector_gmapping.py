@@ -265,11 +265,12 @@ def test_hector_slam_fast_mode_within_contract(pkg, mods):
         assert touched > 1000 and bad <= max(2, touched // 500), (lvl, bad, touched)
 
 
-def test_hector_slam_fast_mode_cluster_match(pkg, mods, monkeypatch):
+def test_hector_slam_fast_mode_cluster_match(pkg, mods):
     """Fast mode spreads the per-point phase of the match over a 4-CTA thread-block cluster (partial sums through
-    distributed shared memory).  Same stream through the clustered and the one-CTA kernel (B2S_HS_CLUSTER=0): poses
-    within the 1e-4 contract of each other and of the CPU processor, identical gate decisions; the clustered path is
-    deterministic (per-scan calls and the one-call stream agree bit for bit)."""
+    distributed shared memory).  Same stream through the clustered kernel and the one-CTA fast match (a batched handle
+    of one processor, hint = previous pose as the stream chains them): poses within the 1e-4 contract of each other and
+    of the CPU processor, identical gate decisions; the clustered path is deterministic (per-scan calls and the one-call
+    stream agree bit for bit)."""
     H, _ = mods
     poses, scans = _stream_case(pkg, H, 33, 60, step_xy=0.1, step_th=3)
     kw = dict(resolution=0.05, size_x=1000, size_y=1000, start=(0.5, 0.5), levels=3, min_dist=0.2, min_angle=0.1)
@@ -277,12 +278,14 @@ def test_hector_slam_fast_mode_cluster_match(pkg, mods, monkeypatch):
     gc = H.HectorSlam(exact=False, **kw)
     if gc.cluster_size() != 4:  # (a device / driver that cannot co-schedule the cooperative grid as clusters: the handle
         pytest.skip("thread-block cluster launch not available here: the fast path runs on one CTA")  # falls back, see hs_create)
-    monkeypatch.setenv("B2S_HS_CLUSTER", "0")
-    g1 = H.HectorSlam(exact=False, **kw)
-    monkeypatch.delenv("B2S_HS_CLUSTER")
-    assert g1.cluster_size() == 1
     pc, uc, _ = gc.process_stream(scans, (0, 0), first_hint=first)
-    p1, u1, _ = g1.process_stream(scans, (0, 0), first_hint=first)
+    g1 = H.HectorSlam(exact=False, batch=1, **kw)
+    est, p1, u1 = first[None], [], []
+    for sc in scans:
+        pb, _, ub = g1.update_batch([sc], (0, 0), est)
+        est = pb.copy()
+        p1.append(pb[0].copy()); u1.append(bool(ub[0]))
+    p1 = np.stack(p1)
     c = port.PortHectorProcessor(**kw)
     est, ref_poses = first, []
     for sc in scans:

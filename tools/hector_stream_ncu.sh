@@ -1,6 +1,5 @@
 OUT=gpurun_out/r2cl
 mkdir -p $OUT
-timeout 200 python tools/hector_cluster_probe.py 2000 > $OUT/probe4.json 2> $OUT/probe4.err
 timeout 500 ncu --set full --clock-control none --import-source on -k regex:k_hs_stream -s 1 -c 1 -o $OUT/hs_stream python tools/hector_stream_ncu.py 300 fast > $OUT/ncu_hs.log 2>&1
 tail -3 $OUT/ncu_hs.log
 if [ -f $OUT/hs_stream.ncu-rep ]; then
