@@ -111,6 +111,14 @@ struct SweepDims {
   int nx = 0, ny = 0, na = 0;
 };
 
+// launch configuration of the last k_sweep_window call (re-run densely when the full volume is asked for)
+struct WinLaunch {
+  int stride = 1;
+  bool gen = false;
+  size_t smem = 0;
+  int ctas = 0, copy_bytes = 0, band_rows = 0, nbands = 1, band_bytes = 0, neg_bands = 0;
+};
+
 }  // namespace b2s
 
 using namespace b2s;
@@ -153,8 +161,19 @@ struct b2s_matcher {
   uint16_t *d_sat = nullptr;  // [B][(sby+1)(sbx+1)] block summed-area tables of the grids
   int sbx = 0, sby = 0;
   bool sat_valid = false;
-  unsigned long long *d_stats = nullptr;  // [0] beam-angle pairs dropped as empty windows in the last sweep
+  unsigned long long *d_stats = nullptr;  // [0] beam-angle pairs dropped as empty windows in the last sweep,
+                                          // [1] (match, angle) pairs k_prune_select kept
   unsigned long long *h_stats = nullptr;  // pinned copy, read back with the results
+  uint8_t *d_mp4 = nullptr;               // [B][mp_pitch] phase-split 4x4 max-pool images (k_grid_mp4)
+  size_t mp_pitch = 0;
+  int mp_guard = 0, mp_lq = 0;
+  bool mp_valid = false;
+  int32_t *d_keep = nullptr, *d_nkeep = nullptr;  // [B][na], [B]: angles a pruned sweep visits
+  size_t keep_cap = 0, nkeep_cap = 0;
+  bool last_pruned = false;  // the last sweep visited only the kept angles: d_sums holds only those
+  bool sums_dense = false;   // d_sums holds every angle of the last sweep
+  WinLaunch win;
+  double last_prune[2] = {1.0, 0.0};
   bool pending = false;                   // a correlate_scan_begin awaits its _end
   int pending_batch = 0;                  // batch size that _begin enqueued
   double last_empty_frac = 0.0;
@@ -550,6 +569,48 @@ __global__ void __launch_bounds__(256)
   for (int i = threadIdx.x; i < (by + 1) * W; i += blockDim.x) out[i] = (uint16_t)s_sat[i];  // < 65536 blocks (checked by the host)
 }
 
+// ----------------------------------------------------------------------------------------------
+// k_grid_mp4: per match, the 4x4 max-pool MP4[j] = max over dy, dx in [0, 4) of grid[j + dy*width_step + dx] in flat
+// index space (zero outside [0, data_size)), for j in [-guard, data_size + guard).  guard >= 3*width_step + 3 + 64, so
+// every j whose pool reaches the grid is covered, including origins just below flat index 0, and the first 12 bytes of
+// phase 0 are zero (k_prune_select redirects rows outside the image there).  k_prune_select reads the
+// pool values of the 8 block columns of one beam row, j + 4*bx, as 8 consecutive bytes: the image is stored split into
+// four column phases, phase p = (j + guard) & 3 at byte p*lq + ((j + guard) >> 2).  One thread per 16 flat bytes
+// (one 32-bit word of each phase); guard % 16 == 0 and width_step % 8 == 0 keep every grid read word-aligned.
+// ----------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256)
+    k_grid_mp4(const uint8_t *__restrict__ grids, size_t grid_pitch, int data_size, int width_step, int guard, int lq,
+               uint8_t *__restrict__ mp_all, size_t mp_pitch) {
+  const int b = blockIdx.y;
+  const int w = blockIdx.x * blockDim.x + threadIdx.x;
+  if (w >= lq / 4) return;
+  const uint8_t *grid = grids + (size_t)b * grid_pitch;
+  const int j = 16 * w - guard;
+  uint32_t o[4] = {0u, 0u, 0u, 0u};  // pool bytes of flat j + 4k + q (word k, byte q)
+#pragma unroll
+  for (int dy = 0; dy < 4; dy++) {
+    const int r = j + dy * width_step;
+    uint32_t W[5], m1[5];
+#pragma unroll
+    for (int q = 0; q < 5; q++) {
+      const int x = r + 4 * q;
+      W[q] = (x >= 0 && x < data_size) ? __ldg(reinterpret_cast<const uint32_t *>(grid + x)) : 0u;
+    }
+#pragma unroll
+    for (int q = 0; q < 5; q++) m1[q] = __vmaxu4(W[q], __funnelshift_r(W[q], q < 4 ? W[q + 1] : 0u, 8));  // max of bytes i, i+1
+#pragma unroll
+    for (int k = 0; k < 4; k++) o[k] = __vmaxu4(o[k], __vmaxu4(m1[k], __funnelshift_r(m1[k], m1[k + 1], 16)));  // i .. i+3
+  }
+  // 4x4 byte transpose: phase p's word w holds byte p of o[0..3]
+  const uint32_t t01l = __byte_perm(o[0], o[1], 0x5140), t01h = __byte_perm(o[0], o[1], 0x7362);
+  const uint32_t t23l = __byte_perm(o[2], o[3], 0x5140), t23h = __byte_perm(o[2], o[3], 0x7362);
+  uint8_t *mp = mp_all + (size_t)b * mp_pitch + 4 * (size_t)w;
+  *reinterpret_cast<uint32_t *>(mp) = __byte_perm(t01l, t23l, 0x5410);
+  *reinterpret_cast<uint32_t *>(mp + lq) = __byte_perm(t01l, t23l, 0x7632);
+  *reinterpret_cast<uint32_t *>(mp + 2 * (size_t)lq) = __byte_perm(t01h, t23h, 0x5410);
+  *reinterpret_cast<uint32_t *>(mp + 3 * (size_t)lq) = __byte_perm(t01h, t23h, 0x7632);
+}
+
 // One block per (match, chunk of OFF_CHUNK angles): window origins grouped as [I0 I1 I2 I3 E0 E1 E2 E3] (I = interior,
 // E = edge, index = a & 3), every group a multiple of 4 long (an interior group donates its 0..3 surplus beams to its edge
 // group; edge groups are padded with far-negative sentinels of the same alignment).  counts[8] holds the group lengths.
@@ -875,6 +936,8 @@ struct ReduceArgs {
   const double *glob_best;
   double *tie_out;
   const double *tie_in;
+  const int32_t *keep;   // [B][na] angles left by k_prune_select (nullptr: every angle)
+  const int32_t *nkeep;  // [B]
 };
 
 
@@ -884,11 +947,13 @@ __global__ void __launch_bounds__(WIN_THREADS, 1)
                    const int32_t *__restrict__ lists, const int32_t *__restrict__ counts,
                    const int32_t *__restrict__ starts, const int32_t *__restrict__ flags, int batch, int n, int na,
                    int nx, int ny, int width_step, int32_t *__restrict__ sums, int *__restrict__ work_counter,
-                   int band_rows, int nbands, int band_bytes, int neg_bands) {
+                   int band_rows, int nbands, int band_bytes, int neg_bands, const int32_t *__restrict__ keep,
+                   const int32_t *__restrict__ nkeep) {
   // Grids larger than shared memory are swept in `nbands` row bands: a work unit is (match, band, 32-row candidate
   // tile); the image holds the rows that tile of a window whose ORIGIN lies in the band can touch (band_rows +
   // STRIDE * 31 + 2), k_offsets_sorted grouped the beams by the band of their origin (bands [0, neg_bands) hold origins
   // BELOW the grid, whose upper tiles still reach it), and the partial sums of the bands are combined with RED.ADD.
+  // keep != nullptr: only the angles keep[b][0 .. nkeep[b]) of match b are swept (k_prune_select; nbands == 1).
   extern __shared__ __align__(128) unsigned char smem[];
   uint8_t *sgrid = smem;  // [WIN_GUARD zeros][band image][WIN_GUARD zeros]
   __shared__ uint64_t bar;
@@ -900,7 +965,7 @@ __global__ void __launch_bounds__(WIN_THREADS, 1)
   constexpr int CPT = 32 / STRIDE;  // candidates per tile row (a tile row is always 32 bytes)
   const int tiles_x = (nx + CPT - 1) / CPT, tiles_y = (ny + 31) >> 5;
   const int unit_tiles_y = nbands > 1 ? tiles_y : 1;        // banded: one row tile per unit
-  const int items = na * tiles_x * (nbands > 1 ? 1 : tiles_y);
+  const int tiles_per_angle = tiles_x * (nbands > 1 ? 1 : tiles_y);
   // word rotation of this lane (see win_load): lanes whose rows start in the same bank get different rotations
   int hi_half = lane >> 4;
   int loff[8];
@@ -965,6 +1030,7 @@ __global__ void __launch_bounds__(WIN_THREADS, 1)
     const int bias = WIN_GUARD - band_lo;
 
     int32_t *bsums = sums + (size_t)b * na * nx * ny;
+    const int items = (keep ? nkeep[b] : na) * tiles_per_angle;
     while (true) {
       int item = 0;
       if (lane == 0) item = atomicAdd(&s_item, 1);
@@ -978,6 +1044,7 @@ __global__ void __launch_bounds__(WIN_THREADS, 1)
         const int t = item % (tiles_x * tiles_y);
         ty = t / tiles_x; tx = t % tiles_x;
       }
+      if (keep) k = keep[(size_t)b * na + k];
       const int row_delta = STRIDE * (ty * 32 + lane) * width_step + tx * 32;  // this lane's row start relative to a beam's origin
       const int32_t *list = lists + ((size_t)b * na + k) * list_cap;
       const int32_t *cn = counts + ((size_t)b * na + k) * ngroups + band * 8;
@@ -1089,6 +1156,7 @@ __device__ __forceinline__ void reduce_match_body(const int b, const ReduceArgs 
   __shared__ int sorted[RED_MAX_TIES];
   __shared__ double s_best;
   __shared__ double s_mean[3];
+  __shared__ int s_keep[1024];  // angle indices the table-driven passes visit, ascending
   if (tid == 0) { s_err = 0; s_count = 0; }
   if (!s.fine && mode <= 1)
     for (int i = tid; i < pstep * g.search_side; i += RED_THREADS) probs[i] = 0.0;  // Clear (Mapper.cpp:329)
@@ -1109,6 +1177,10 @@ __device__ __forceinline__ void reduce_match_body(const int b, const ReduceArgs 
     }
     s_apf[k] = (float)(apen / D);
   }
+  // a pruned sweep computed only the angles k_prune_select kept; every candidate that can be the best, a tie or a
+  // per-cell maximum the covariance reads lies in one of them (see k_prune_select)
+  const int nk = (tab && A.keep) ? A.nkeep[b] : na;
+  for (int j = tid; j < nk && tab; j += RED_THREADS) s_keep[j] = A.keep ? A.keep[(size_t)b * na + j] : j;
   __syncthreads();
 
   // ---- pass 1: best response + per-cell maxima (Mapper.cpp:430-451); one thread per (x,y) cell ----
@@ -1130,19 +1202,20 @@ __device__ __forceinline__ void reduce_match_body(const int b, const ReduceArgs 
       int kmax = 0;
       int32_t vmax = 0;
       bool near = false, any_amb = false;
-      for (int k0 = 0; k0 < na; k0 += RED_UNROLL) {
+      for (int j0 = 0; j0 < nk; j0 += RED_UNROLL) {
         int32_t v[RED_UNROLL];
 #pragma unroll
-        for (int u = 0; u < RED_UNROLL; u++) v[u] = (k0 + u < na) ? __ldcg(bs + (size_t)(k0 + u) * ncell + c) : 0;
+        for (int u = 0; u < RED_UNROLL; u++) v[u] = (j0 + u < nk) ? __ldcg(bs + (size_t)s_keep[j0 + u] * ncell + c) : 0;
 #pragma unroll
         for (int u = 0; u < RED_UNROLL; u++) {
-          if (k0 + u >= na) continue;
+          if (j0 + u >= nk) continue;
+          const int k = s_keep[j0 + u];
           bool amb;
-          const float f = red_fscore(v[u], s_apf[k0 + u], dpf, inv_d, pen, amb);
+          const float f = red_fscore(v[u], s_apf[k], dpf, inv_d, pen, amb);
           any_amb |= amb;
           if (f > fmax) {
             near = fmax >= f * (1.0f - 2.0e-6f) - 1.0e-30f;  // the old maximum (and only it or its own near ones) may still be near
-            fmax = f; kmax = k0 + u; vmax = v[u];
+            fmax = f; kmax = k; vmax = v[u];
           } else if (f >= fmax * (1.0f - 2.0e-6f) - 1.0e-30f) {
             near = true;
           }
@@ -1157,17 +1230,18 @@ __device__ __forceinline__ void reduce_match_body(const int b, const ReduceArgs 
         cell_best = 0.0;  // every sum is 0: response 0 / D, never penalised (Mapper.cpp:399)
       } else {
         const float thr = fmax * (1.0f - 2.0e-6f) - 1.0e-30f;
-        for (int k0 = 0; k0 < na; k0 += RED_UNROLL) {
+        for (int j0 = 0; j0 < nk; j0 += RED_UNROLL) {
           int32_t v[RED_UNROLL];
 #pragma unroll
-          for (int u = 0; u < RED_UNROLL; u++) v[u] = (k0 + u < na) ? __ldcg(bs + (size_t)(k0 + u) * ncell + c) : 0;
+          for (int u = 0; u < RED_UNROLL; u++) v[u] = (j0 + u < nk) ? __ldcg(bs + (size_t)s_keep[j0 + u] * ncell + c) : 0;
 #pragma unroll
           for (int u = 0; u < RED_UNROLL; u++) {
-            if (k0 + u >= na) continue;
+            if (j0 + u >= nk) continue;
+            const int k = s_keep[j0 + u];
             bool amb;
-            const float f = red_fscore(v[u], s_apf[k0 + u], dpf, inv_d, pen, amb);
+            const float f = red_fscore(v[u], s_apf[k], dpf, inv_d, pen, amb);
             if (f >= thr || amb) {
-              const double angle = start_a + (double)(uint32_t)(k_first + k0 + u) * s.angle_res;
+              const double angle = start_a + (double)(uint32_t)(k_first + k) * s.angle_res;
               cell_best = dmax(cell_best, candidate_response(v[u], n, pen, sq, angle, ch, p));
             }
           }
@@ -1219,14 +1293,15 @@ __device__ __forceinline__ void reduce_match_body(const int b, const ReduceArgs 
     const double y = start_y + (double)(uint32_t)iy * s.res_y, x = start_x + (double)(uint32_t)ix * s.res_x;
     const double sq = x * x + y * y;
     const float dpf = (float)dmax(1.0 - (DISTANCE_PENALTY_GAIN * sq / p.distance_variance_penalty), p.minimum_distance_penalty);
-    for (int k0 = 0; k0 < na; k0 += RED_UNROLL) {
+    for (int j0 = 0; j0 < nk; j0 += RED_UNROLL) {
       int32_t v[RED_UNROLL];
 #pragma unroll
-      for (int u = 0; u < RED_UNROLL; u++) v[u] = (k0 + u < na) ? __ldcg(bs + (size_t)(k0 + u) * ncell + c) : 0;
+      for (int u = 0; u < RED_UNROLL; u++)
+        v[u] = (j0 + u < nk) ? __ldcg(bs + (size_t)(tab ? s_keep[j0 + u] : j0 + u) * ncell + c) : 0;
 #pragma unroll
       for (int u = 0; u < RED_UNROLL; u++) {
-        const int k = k0 + u;
-        if (k >= na) continue;
+        if (j0 + u >= nk) continue;
+        const int k = tab ? s_keep[j0 + u] : j0 + u;
         if (tab) {
           bool amb;
           const float f = red_fscore(v[u], s_apf[k], dpf, inv_d, pen, amb);
@@ -1382,6 +1457,220 @@ __global__ void __launch_bounds__(RED_THREADS, 2) k_reduce(ReduceArgs A) {
 }
 
 // ----------------------------------------------------------------------------------------------
+// k_prune_select: which angles of a stride-1, one-tile (nx, ny <= 32) window sweep can change a result.  One CTA per
+// match, the phase-split 4x4 max-pool image (k_grid_mp4) staged into shared memory by TMA bulk copy.
+//
+// 1. Bound.  For angle k and 4x4 candidate block (by, bx), every candidate's integer sum is at most
+//    S(k, by, bx) = sum over the listed beams i of MP4[a_i + 4*by*width_step + 4*bx]  (a_i = window origin).  Beams
+//    k_offsets_sorted dropped as empty windows add 0 to every exact sum and are left out here too.  The penalised bound
+//    applies the reference's fp64 operations to S, the block's largest distance penalty and the angle's penalty;
+//    correctly rounded operations are monotone, so it is >= every candidate's response.  A candidate whose unpenalised
+//    response is within KT_TOLERANCE of 0 is not penalised (Mapper.cpp:399): it is <= min(S / (N*100), 1.1e-6).
+//    Warps pull angles; lane = (beam group g, block row by); a beam row's 8 block columns are 8 consecutive bytes of
+//    one phase, summed as packed u16 lanes.  bound[k] = max over the angle's blocks; the top (bound, angle, block)
+//    is kept with a packed 64-bit atomicMax.
+// 2. Seed.  The 16 candidates of the top block are evaluated exactly (same fp64 operations as k_reduce); their
+//    maximum L is a response of the volume, so L <= best.
+// 3. Select.  Angle k is kept iff bound[k] >= L - 0.1 - 1e-9 (the 1e-9 only ever keeps more).
+// Why the results are unchanged: the outputs of CorrelateScan depend on the best response, on the candidates within
+// KT_TOLERANCE of it (the ties, summed in (y, x, theta) order) and, for the covariance, on the per-cell maxima over
+// angles of the cells whose maximum is >= best - 0.1 (ComputePositionalCovariance, Mapper.cpp:586).  Each of these is a
+// candidate with response >= best - 0.1 >= L - 0.1, so its block bound, and hence its angle's bound, clears the cut:
+// its angle is kept.  So the best, the tie set and its order, and every per-cell maximum the covariance reads come out
+// identical when k_sweep_window and k_reduce visit only the kept angles.  A cell whose true maximum is below the cut
+// may get a smaller partial maximum, but it is excluded either way.  (When best < 0.1 every bound clears the cut.)
+// Irregular lattices (k_sweep_generic sweeps every angle) keep every angle; out-of-range lattices keep none.
+// ----------------------------------------------------------------------------------------------
+constexpr int PRUNE_THREADS = 512;
+constexpr double PRUNE_CUT = 0.1;     // ComputePositionalCovariance's window below the best response
+constexpr double PRUNE_EPS = 1e-9;    // guard against rounding in the bound product
+__global__ void __launch_bounds__(PRUNE_THREADS, 1)
+    k_prune_select(const uint8_t *__restrict__ mp_all, size_t mp_pitch, int lq, int mp_guard,
+                   const uint8_t *__restrict__ grids, size_t grid_pitch, int data_size, int width_step,
+                   const int32_t *__restrict__ lists, const int32_t *__restrict__ counts,
+                   const int32_t *__restrict__ starts, const int32_t *__restrict__ flags,
+                   const double *__restrict__ centers, b2s_matcher_params p, b2s_search s, int n, int na, int nx,
+                   int ny, int32_t *__restrict__ keep, int32_t *__restrict__ nkeep,
+                   unsigned long long *__restrict__ stats) {
+  extern __shared__ __align__(128) unsigned char smp[];  // [4][lq] phase-split MP4 image
+  __shared__ uint64_t bar;
+  __shared__ double s_ab[1024];     // per-angle bound
+  __shared__ double s_dp[64];       // per-block largest distance penalty
+  __shared__ double s_cand[16];     // exact responses of the top block's candidates
+  __shared__ unsigned long long s_top;
+  __shared__ int s_wc[PRUNE_THREADS / 32], s_kept;
+  const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int f = flags[b];
+  if ((f & 2) || !(f & 1)) {
+    const int nk = (f & 2) ? 0 : na;  // irregular: k_sweep_generic sweeps every angle, k_reduce reads every angle
+    for (int k = tid; k < nk; k += PRUNE_THREADS) keep[(size_t)b * na + k] = k;
+    if (tid == 0) {
+      nkeep[b] = nk;
+      if (nk) atomicAdd(stats + 1, (unsigned long long)nk);
+    }
+    return;
+  }
+  const int mp_bytes = 4 * lq;
+  if (tid == 0) {
+    mbar_init(&bar, 1);
+    fence_mbar_init();
+    s_top = 0ull;
+    s_kept = 0;
+  }
+  __syncthreads();
+  if (tid == 0) {
+    mbar_expect_tx(&bar, (uint32_t)mp_bytes);
+    const uint8_t *src = mp_all + (size_t)b * mp_pitch;
+    for (int off = 0; off < mp_bytes; off += 32768) bulk_g2s(smp + off, src + off, (uint32_t)min(32768, mp_bytes - off), &bar);
+  }
+  const bool pen = s.do_penalize != 0;
+  const double ch = centers[3 * b + 2];
+  const double start_x = -s.offset_x, start_y = -s.offset_y, start_a = ch - s.angle_offset;
+  const int nbx = (nx + 3) >> 2, nby = (ny + 3) >> 2;
+  if (tid < 64) {
+    const int by = tid >> 3, bx = tid & 7;
+    double dp = 0.0;
+    for (int dy = 0; dy < 4; dy++)
+      for (int dx = 0; dx < 4; dx++) {
+        const int iy = 4 * by + dy, ix = 4 * bx + dx;
+        if (iy >= ny || ix >= nx) continue;
+        const double y = start_y + (double)(uint32_t)iy * s.res_y, x = start_x + (double)(uint32_t)ix * s.res_x;
+        const double sq = x * x + y * y;
+        dp = dmax(dp, dmax(1.0 - (DISTANCE_PENALTY_GAIN * sq / p.distance_variance_penalty), p.minimum_distance_penalty));
+      }
+    s_dp[tid] = dp;
+  }
+  mbar_wait(&bar, 0);
+  __syncthreads();
+
+  // ---- 1. bounds ----
+  const int list_cap = n + LIST_PAD;
+  const double D = (double)((uint32_t)n * (uint32_t)GRID_OCCUPIED);
+  const int g = lane >> 3, by = lane & 7;
+  const uint32_t row_off = (uint32_t)(4 * by * width_step + mp_guard);
+  const uint32_t lim = (uint32_t)(data_size + 2 * mp_guard - 32);  // a row starting above lim reads only zero pool values
+  for (int k = warp; k < na; k += PRUNE_THREADS / 32) {
+    const size_t bk = (size_t)b * na + k;
+    const int32_t *list = lists + bk * list_cap;
+    const int total = starts[bk * 8 + 7] + counts[bk * 8 + 7];  // the 8 groups are contiguous
+    uint32_t e0 = 0, o0 = 0, e1 = 0, o1 = 0;  // packed u16: block columns (0, 2), (1, 3), (4, 6), (5, 7)
+    uint32_t sum[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+    auto flush = [&]() {
+      sum[0] += e0 & 0xffffu; sum[2] += e0 >> 16; sum[1] += o0 & 0xffffu; sum[3] += o0 >> 16;
+      sum[4] += e1 & 0xffffu; sum[6] += e1 >> 16; sum[5] += o1 & 0xffffu; sum[7] += o1 >> 16;
+      e0 = o0 = e1 = o1 = 0;
+    };
+    int chunks = 0;
+    for (int ib = 0; ib < total; ib += 32) {
+      const int32_t mine = (ib + lane < total) ? __ldg(list + ib + lane) : WIN_SKIP;
+#pragma unroll
+      for (int jj = 0; jj < 8; jj++) {
+        uint32_t u = (uint32_t)__shfl_sync(0xffffffffu, mine, jj * 4 + g) + row_off;
+        // below -mp_guard or past data_size + mp_guard - 32 every pool value of the row is 0: read the zero-valued
+        // start of phase 0 instead (branch-free, so the unrolled beams' loads overlap)
+        u = u <= lim ? u : 0u;
+        const uint32_t t = u >> 2, sh = (t & 3) * 8;
+        const uint32_t *w = reinterpret_cast<const uint32_t *>(smp + (u & 3) * lq + (t & ~3u));
+        const uint32_t w0 = w[0], w1 = w[1], w2 = w[2];
+        const uint32_t lo = __funnelshift_r(w0, w1, sh), hi = __funnelshift_r(w1, w2, sh);
+        e0 += lo & 0x00ff00ffu; o0 += (lo >> 8) & 0x00ff00ffu;
+        e1 += hi & 0x00ff00ffu; o1 += (hi >> 8) & 0x00ff00ffu;
+      }
+      if (++chunks == 64) { flush(); chunks = 0; }  // 64 x 8 beams x 127 < 65536
+    }
+    flush();
+#pragma unroll
+    for (int q = 0; q < 8; q++) {
+      sum[q] += __shfl_xor_sync(0xffffffffu, sum[q], 8);
+      sum[q] += __shfl_xor_sync(0xffffffffu, sum[q], 16);
+    }
+    const double angle = start_a + (double)(uint32_t)k * s.angle_res;
+    const double apen = dmax(1.0 - (ANGLE_PENALTY_GAIN * ((angle - ch) * (angle - ch)) / p.angle_variance_penalty),
+                             p.minimum_angle_penalty);
+    double bk_best = -1.0;
+    unsigned long long key = 0ull;
+    if (g == 0 && by < nby) {
+#pragma unroll
+      for (int bx = 0; bx < 8; bx++) {
+        if (bx >= nbx) continue;
+        const double r = (double)sum[bx] / D;
+        const double bd = pen ? dmax(r * (s_dp[by * 8 + bx] * apen), r < 1.1e-6 ? r : 1.1e-6) : r;
+        if (bd > bk_best) {
+          bk_best = bd;
+          key = ((unsigned long long)__double_as_longlong(bd) & ~0xffffull) | (unsigned long long)((k << 6) | (by << 3) | bx);
+        }
+      }
+    }
+#pragma unroll
+    for (int d = 4; d > 0; d >>= 1) {
+      bk_best = dmax(bk_best, __shfl_xor_sync(0xffffffffu, bk_best, d));
+      const unsigned long long o = __shfl_xor_sync(0xffffffffu, key, d);
+      key = o > key ? o : key;
+    }
+    if (lane == 0) {
+      s_ab[k] = bk_best;
+      atomicMax(&s_top, key);
+    }
+  }
+  __syncthreads();
+
+  // ---- 2. seed: the top block's candidates, exactly ----
+  {
+    const unsigned long long key = s_top;
+    const int k = (int)((key >> 6) & 1023), tby = (int)((key >> 3) & 7), tbx = (int)(key & 7);
+    const int iy = 4 * tby + (warp >> 2), ix = 4 * tbx + (warp & 3);  // 16 warps, one candidate each
+    const bool valid = iy < ny && ix < nx;
+    int32_t isum = 0;
+    if (valid) {
+      const size_t bk = (size_t)b * na + k;
+      const int32_t *list = lists + bk * list_cap;
+      const int total = starts[bk * 8 + 7] + counts[bk * 8 + 7];
+      const uint8_t *grid = grids + (size_t)b * grid_pitch;
+      const int32_t rel = iy * width_step + ix;
+      for (int i = lane; i < total; i += 32) {
+        const int32_t idx = (int32_t)((uint32_t)__ldg(list + i) + (uint32_t)rel);
+        if ((uint32_t)idx < (uint32_t)data_size) isum += grid[idx];
+      }
+    }
+#pragma unroll
+    for (int d = 16; d > 0; d >>= 1) isum += __shfl_xor_sync(0xffffffffu, isum, d);
+    if (lane == 0) {
+      double r = -1.0;
+      if (valid) {
+        const double y = start_y + (double)(uint32_t)iy * s.res_y, x = start_x + (double)(uint32_t)ix * s.res_x;
+        r = candidate_response(isum, n, pen, x * x + y * y, start_a + (double)(uint32_t)k * s.angle_res, ch, p);
+      }
+      s_cand[warp] = r;
+    }
+  }
+  __syncthreads();
+  double L = s_cand[0];
+  for (int i = 1; i < 16; i++) L = dmax(L, s_cand[i]);
+  const double cut = L - PRUNE_CUT - PRUNE_EPS;
+
+  // ---- 3. select: compact the kept angles in ascending order ----
+  for (int k0 = 0; k0 < na; k0 += PRUNE_THREADS) {
+    const int k = k0 + tid;
+    const bool kp = k < na && s_ab[k] >= cut;
+    const unsigned bal = __ballot_sync(0xffffffffu, kp);
+    if (lane == 0) s_wc[warp] = __popc(bal);
+    __syncthreads();
+    int off = s_kept;
+    for (int w = 0; w < warp; w++) off += s_wc[w];
+    off += __popc(bal & ((1u << lane) - 1u));
+    if (kp) keep[(size_t)b * na + off] = k;
+    __syncthreads();
+    if (tid == 0)
+      for (int w = 0; w < PRUNE_THREADS / 32; w++) s_kept += s_wc[w];
+    __syncthreads();
+  }
+  if (tid == 0) {
+    nkeep[b] = s_kept;
+    atomicAdd(stats + 1, (unsigned long long)s_kept);
+  }
+}
+
+// ----------------------------------------------------------------------------------------------
 // k_angular_cov: ComputeAngularCovariance (Mapper.cpp:641-692).  One CTA per match; warps over angles,
 // lanes over beams (GetResponse at the best cell), then thread 0 accumulates in angle order.
 // ----------------------------------------------------------------------------------------------
@@ -1518,8 +1807,58 @@ static b2s_status ensure_cap(T **p, size_t *cap, size_t count) {
 static b2s_status run_correlate(b2s_matcher *m, const b2s_search *s, bool centers_on_device, int k_first = 0,
                                 int na_override = -1, int mode = 0);
 
-// (re)build the per-match block summed-area tables after the grids changed
+// k_sweep_window over the lists of the last lookup stage with m->win's configuration; pruned: only the kept angles
+static b2s_status launch_window(b2s_matcher *m, int B, int n, int na, int nx, int ny, bool pruned) {
+  const WinLaunch &w = m->win;
+  B2S_CUDA_CHECK(cudaMemsetAsync(m->d_work, 0, sizeof(int), m->stream));
+  if (w.nbands > 1)  // bands accumulate with RED.ADD
+    B2S_CUDA_CHECK(cudaMemsetAsync(m->d_sums, 0, sizeof(int32_t) * (size_t)B * na * nx * ny, m->stream));
+  auto launch = [&](auto kern) -> b2s_status {
+    B2S_CUDA_CHECK(raise_dyn_smem(kern, w.smem));
+    kern<<<w.ctas, WIN_THREADS, w.smem, m->stream>>>(m->d_grids, m->grid_pitch, m->g.data_size, w.copy_bytes, m->d_lists,
+                                                     m->d_counts, m->d_starts, m->d_flags, B, n, na, nx, ny,
+                                                     m->g.width_step, m->d_sums, m->d_work, w.band_rows, w.nbands,
+                                                     w.band_bytes, w.neg_bands, pruned ? m->d_keep : nullptr,
+                                                     pruned ? m->d_nkeep : nullptr);
+    return B2S_OK;
+  };
+  if (w.stride == 2) return w.gen ? launch(k_sweep_window<2, true>) : launch(k_sweep_window<2, false>);
+  return w.gen ? launch(k_sweep_window<1, true>) : launch(k_sweep_window<1, false>);
+}
+
+// (re)build the per-match max-pool images k_prune_select stages into shared memory, when one fits there
+static b2s_status build_mp4(b2s_matcher *m) {
+  m->mp_valid = false;
+  const b2s_grid_info &g = m->g;
+  if (g.width_step % 8 != 0 || m->grid_high_bytes) return B2S_OK;  // no pruned sweep
+  // >= 3*width_step + 3 + 32 (see k_grid_mp4) and > 3*width_step + 47: phase 0's first 12 bytes pool no grid cell
+  m->mp_guard = (3 * g.width_step + 3 + 64 + 15) & ~15;
+  m->mp_lq = ((g.data_size + 2 * m->mp_guard) / 4 + 16 + 15) & ~15;
+  static size_t prune_static = 0;
+  if (!prune_static) {
+    cudaFuncAttributes fa;
+    B2S_CUDA_CHECK(cudaFuncGetAttributes(&fa, k_prune_select));
+    prune_static = fa.sharedSizeBytes;
+  }
+  const size_t bytes = 4 * (size_t)m->mp_lq;
+  if (bytes + prune_static + 512 > (size_t)m->smem_optin) return B2S_OK;
+  if (!m->d_mp4) {
+    m->mp_pitch = (bytes + 127) & ~(size_t)127;
+    b2s_status st = dev_alloc(&m->d_mp4, (size_t)m->max_batch * m->mp_pitch);
+    if (st) return st;
+  }
+  const dim3 grid((unsigned)ceil_div(m->mp_lq / 4, 256), (unsigned)m->batch);
+  k_grid_mp4<<<grid, 256, 0, m->stream>>>(m->d_grids, m->grid_pitch, g.data_size, g.width_step, m->mp_guard, m->mp_lq,
+                                          m->d_mp4, m->mp_pitch);
+  B2S_CUDA_CHECK(cudaGetLastError());
+  m->mp_valid = true;
+  return B2S_OK;
+}
+
+// (re)build the per-match block summed-area tables and max-pool images after the grids changed
 static b2s_status build_sat(b2s_matcher *m) {
+  b2s_status st = build_mp4(m);
+  if (st) return st;
   const size_t sm = sizeof(uint32_t) * (size_t)(m->sbx + 1) * (m->sby + 1);
   m->sat_valid = false;
   if (sm > 200 * 1024 || (m->g.width_step % 4) != 0 || (long long)m->sbx * m->sby >= 65535) return B2S_OK;  // no skipping
@@ -1599,14 +1938,14 @@ static b2s_status matcher_create_impl(const b2s_matcher_params *params, const b2
   m->sbx = (g.width_step + 3) / 4;
   m->sby = (g.height + 3) / 4;
   if ((st = dev_alloc(&m->d_sat, B * (size_t)((((m->sbx + 1) * (m->sby + 1)) + 7) & ~7)))) return st;  // per-match stride padded to 16 bytes
-  if ((st = dev_alloc(&m->d_stats, 1))) return st;
+  if ((st = dev_alloc(&m->d_stats, 2))) return st;
   if ((st = dev_alloc(&m->d_part_best, B))) return st;
   if ((st = dev_alloc(&m->d_glob_best, B))) return st;
   if ((st = dev_alloc(&m->d_tie, B * 5))) return st;
   if ((st = dev_alloc(&m->d_status, B))) return st;
   B2S_CUDA_CHECK(cudaMallocHost(reinterpret_cast<void **>(&m->h_results), B * sizeof(b2s_match_result)));
-  B2S_CUDA_CHECK(cudaMallocHost(reinterpret_cast<void **>(&m->h_stats), sizeof(unsigned long long)));
-  *m->h_stats = 0;
+  B2S_CUDA_CHECK(cudaMallocHost(reinterpret_cast<void **>(&m->h_stats), 2 * sizeof(unsigned long long)));
+  m->h_stats[0] = m->h_stats[1] = 0;
   B2S_CUDA_CHECK(cudaMemsetAsync(m->d_grids, 0, B * m->grid_pitch, m->stream));
   B2S_CUDA_CHECK(cudaMemsetAsync(m->d_results, 0, B * sizeof(b2s_match_result), m->stream));
   B2S_CUDA_CHECK(cudaStreamSynchronize(m->stream));
@@ -1642,7 +1981,7 @@ void b2s_matcher_destroy(b2s_matcher *m) {
   cudaSetDevice(m->device);
   if (m->stream) cudaStreamSynchronize(m->stream);
   void *ptrs[] = {m->d_kernel, m->d_ranges, m->d_poses, m->d_sensor, m->d_pts, m->d_local, m->d_grids,
-                  m->d_grid_off, m->d_base_ranges, m->d_base_poses, m->d_base_pts, m->d_pool, m->d_base_src, m->d_lut, m->d_lists, m->d_counts, m->d_starts, m->d_sat, m->d_stats, m->d_part_best, m->d_glob_best, m->d_tie, m->d_status, m->d_sums, m->d_bases,
+                  m->d_grid_off, m->d_base_ranges, m->d_base_poses, m->d_base_pts, m->d_pool, m->d_base_src, m->d_lut, m->d_lists, m->d_counts, m->d_starts, m->d_sat, m->d_stats, m->d_mp4, m->d_keep, m->d_nkeep, m->d_part_best, m->d_glob_best, m->d_tie, m->d_status, m->d_sums, m->d_bases,
                   m->d_flags, m->d_probs, m->d_centers, m->d_results, m->d_work};
   for (void *p : ptrs)
     if (p) cudaFree(p);
@@ -1875,7 +2214,7 @@ b2s_status b2s_matcher_correlate_scan_begin(b2s_matcher *m, const double *center
   b2s_status st = run_correlate(m, search, true);
   if (st) return st;
   B2S_CUDA_CHECK(cudaMemcpyAsync(m->h_results, m->d_results, sizeof(b2s_match_result) * B, cudaMemcpyDeviceToHost, m->stream));
-  B2S_CUDA_CHECK(cudaMemcpyAsync(m->h_stats, m->d_stats, sizeof(unsigned long long), cudaMemcpyDeviceToHost, m->stream));
+  B2S_CUDA_CHECK(cudaMemcpyAsync(m->h_stats, m->d_stats, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, m->stream));
   m->pending = true;
   m->pending_batch = B;
   return B2S_OK;
@@ -1891,6 +2230,9 @@ b2s_status b2s_matcher_correlate_scan_end(b2s_matcher *m, b2s_match_result *resu
   std::memcpy(results, m->h_results, sizeof(b2s_match_result) * B);
   if (m->last_path == 2 && m->last.na > 0 && m->n > 0) m->last_empty_frac = (double)*m->h_stats / ((double)B * m->last.na * m->n);
   else m->last_empty_frac = 0.0;
+  const double pairs = (double)B * m->last.na;
+  if (m->last_pruned) { m->last_prune[0] = pairs > 0 ? (double)m->h_stats[1] / pairs : 1.0; m->last_prune[1] = (double)m->h_stats[1]; }
+  else { m->last_prune[0] = 1.0; m->last_prune[1] = pairs; }
   for (int i = 1; i < 3; i++) {
     float ms = 0;
     if (cudaEventElapsedTime(&ms, m->ev[i - 1], m->ev[i]) == cudaSuccess) m->last_ms[i - 1] = ms;
@@ -2036,6 +2378,7 @@ static ReduceArgs reduce_args(b2s_matcher *m, const b2s_search &s, int nx, int n
   A.probs_all = m->d_probs; A.results = m->d_results;
   A.k_first = k_first; A.mode = mode;
   A.part_best = m->d_part_best; A.glob_best = m->d_glob_best; A.tie_out = m->d_tie; A.tie_in = m->d_tie;
+  A.keep = nullptr; A.nkeep = nullptr;
   return A;
 }
 
@@ -2150,6 +2493,12 @@ b2s_status b2s_matcher_get_response_sums(b2s_matcher *m, int b, int32_t *out, in
   if (!m->have_sweep) B2S_FAIL(B2S_ERR_BAD_STATE, "no sweep has been run");
   B2S_CUDA_CHECK(cudaSetDevice(m->device));
   const int nx = m->last.nx, ny = m->last.ny, na = m->last.na;
+  if (!m->sums_dense) {  // a pruned sweep left the other angles unswept: sweep every angle once from the held lists
+    b2s_status st = launch_window(m, m->batch, m->n, na, nx, ny, false);
+    if (st) return st;
+    B2S_CUDA_CHECK(cudaGetLastError());
+    m->sums_dense = true;
+  }
   std::vector<int32_t> tmp((size_t)nx * ny * na);
   B2S_CUDA_CHECK(cudaMemcpyAsync(tmp.data(), m->d_sums + (size_t)b * nx * ny * na, sizeof(int32_t) * tmp.size(),
                                  cudaMemcpyDeviceToHost, m->stream));
@@ -2167,6 +2516,13 @@ b2s_status b2s_matcher_last_stats(b2s_matcher *m, double out[4]) {
   out[1] = (double)m->last_path;
   out[2] = (double)m->last.na * m->last.nx * m->last.ny;
   out[3] = (double)m->n;
+  return B2S_OK;
+}
+
+b2s_status b2s_matcher_last_prune_stats(b2s_matcher *m, double out[2]) {
+  if (!m || !out) B2S_FAIL(B2S_ERR_BAD_PARAMS, "null argument");
+  out[0] = m->last_prune[0];
+  out[1] = m->last_prune[1];
   return B2S_OK;
 }
 
@@ -2269,7 +2625,7 @@ static b2s_status run_correlate(b2s_matcher *m, const b2s_search *s, bool /*cent
     if ((((size_t)n * OFF_SMEM_PER_BEAM + 15) & ~(size_t)15) + sizeof(uint16_t) * (size_t)((((m->sbx + 1) * (m->sby + 1)) + 7) & ~7) + 64 > 200 * 1024) skip_empty = false;
     const size_t sat_bytes = skip_empty ? sizeof(uint16_t) * (size_t)((((m->sbx + 1) * (m->sby + 1)) + 7) & ~7) : 0;
     const size_t osm = (((size_t)n * OFF_SMEM_PER_BEAM + 15) & ~(size_t)15) + sat_bytes + 64;
-    B2S_CUDA_CHECK(cudaMemsetAsync(m->d_stats, 0, sizeof(unsigned long long), m->stream));
+    B2S_CUDA_CHECK(cudaMemsetAsync(m->d_stats, 0, 2 * sizeof(unsigned long long), m->stream));
     if (osm > 16 * 1024)  // static + dynamic shared memory together must stay under the 48 KB default: opt in early
       B2S_CUDA_CHECK(raise_dyn_smem(k_offsets_sorted, osm));
     k_offsets_sorted<<<B * ((na + OFF_CHUNK - 1) / OFF_CHUNK), 256, osm, m->stream>>>(
@@ -2282,31 +2638,39 @@ static b2s_status run_correlate(b2s_matcher *m, const b2s_search *s, bool /*cent
   B2S_CUDA_CHECK(cudaEventRecord(m->ev[1], m->stream));
 
   // ---- response sweep ----
+  // Pruned sweep (k_prune_select): only the angles that can change a result are swept.  It covers the one-tile,
+  // stride-1, whole-grid window sweep of a complete coarse-stage CorrelateScan; kernel selector 3 keeps the dense sweep.
+  const bool prune = use_window && na > 0 && m->force_kernel != 3 && m->mp_valid && stride == 1 && nbands == 1 &&
+                     !s->fine && k_first == 0 && na == na_full && mode == 0 && nx <= 32 && ny <= 32 && na <= 1024;
+  m->last_pruned = prune;
+  m->sums_dense = !prune;
   if (na == 0) {
     m->last_path = use_window ? 2 : 1;  // empty angle subset of a split sweep: nothing to sweep
   } else if (use_window) {
-    B2S_CUDA_CHECK(cudaMemsetAsync(m->d_work, 0, sizeof(int), m->stream));
-    if (nbands > 1)  // bands accumulate with RED.ADD
-      B2S_CUDA_CHECK(cudaMemsetAsync(m->d_sums, 0, sizeof(int32_t) * (size_t)B * na * ncell, m->stream));
-    const int ctas = (int)std::min<long long>((long long)B * nbands * (nbands > 1 ? tiles_y_w : 1), m->num_sms);
     // (A variant that ran each match's fp64 tail inside the sweep CTA right after its last tile — volume read back from
     // L2, no k_reduce pass — was built, parity-tested and measured SLOWER on cfg 2, 8.80 -> 9.06 ms per 1024 matches: the
     // sweep kernel owns its SM, so the tail's serial stretches are no longer hidden by a second resident CTA as they are
     // in the stand-alone k_reduce.  Removed again; DESIGN.md §4.)
     // the GEN = false instantiation assumes exactly two lanes per row-start bank (see win_load)
     const int bank_step = ((m->g.width_step >> 2) * std::max(stride, 1)) & 31;
-    const bool gen = (bank_step & 3) != 2;
-    auto launch = [&](auto kern) -> b2s_status {
-      B2S_CUDA_CHECK(raise_dyn_smem(kern, win_smem));
-      kern<<<ctas, WIN_THREADS, win_smem, m->stream>>>(m->d_grids, m->grid_pitch, m->g.data_size, copy_bytes, m->d_lists,
-                                                   m->d_counts, m->d_starts, m->d_flags, B, n, na, nx, ny,
-                                                   m->g.width_step, m->d_sums, m->d_work, band_rows, nbands,
-                                                   band_bytes, neg_bands);
-      return B2S_OK;
-    };
-    if (stride == 2) st = gen ? launch(k_sweep_window<2, true>) : launch(k_sweep_window<2, false>);
-    else st = gen ? launch(k_sweep_window<1, true>) : launch(k_sweep_window<1, false>);
-    if (st) return st;
+    m->win.stride = stride;
+    m->win.gen = (bank_step & 3) != 2;
+    m->win.smem = win_smem;
+    m->win.ctas = (int)std::min<long long>((long long)B * nbands * (nbands > 1 ? tiles_y_w : 1), m->num_sms);
+    m->win.copy_bytes = copy_bytes; m->win.band_rows = band_rows; m->win.nbands = nbands;
+    m->win.band_bytes = band_bytes; m->win.neg_bands = neg_bands;
+    if (prune) {
+      if ((st = ensure_cap(&m->d_keep, &m->keep_cap, (size_t)B * na))) return st;
+      if ((st = ensure_cap(&m->d_nkeep, &m->nkeep_cap, (size_t)B))) return st;
+      const size_t psm = 4 * (size_t)m->mp_lq;
+      B2S_CUDA_CHECK(raise_dyn_smem(k_prune_select, psm));
+      k_prune_select<<<B, PRUNE_THREADS, psm, m->stream>>>(
+          m->d_mp4, m->mp_pitch, m->mp_lq, m->mp_guard, m->d_grids, m->grid_pitch, m->g.data_size, m->g.width_step,
+          m->d_lists, m->d_counts, m->d_starts, m->d_flags, m->d_centers, m->p, *s, n, na, nx, ny, m->d_keep,
+          m->d_nkeep, m->d_stats);
+      B2S_CUDA_CHECK(cudaGetLastError());
+    }
+    if ((st = launch_window(m, B, n, na, nx, ny, prune))) return st;
     // matches whose lattice is not the regular raster (a centre exactly on a rounding tie) fall through;
     // they compute their lookup values on the fly (no table was materialised for them)
     // (a few CTAs per match that exit at once unless the lattice is irregular: the kernel loops over the cells)
@@ -2326,7 +2690,9 @@ static b2s_status run_correlate(b2s_matcher *m, const b2s_search *s, bool /*cent
   B2S_CUDA_CHECK(cudaEventRecord(m->ev[2], m->stream));
 
   // ---- fp64 tail ----
-  k_reduce<<<B, RED_THREADS, 0, m->stream>>>(reduce_args(m, *s, nx, ny, na, k_first, mode));
+  ReduceArgs ra = reduce_args(m, *s, nx, ny, na, k_first, mode);
+  if (prune) { ra.keep = m->d_keep; ra.nkeep = m->d_nkeep; }
+  k_reduce<<<B, RED_THREADS, 0, m->stream>>>(ra);
   if (s->fine) {
     size_t sm = sizeof(double) * (size_t)na;
     if (sm > 48 * 1024) B2S_FAIL(B2S_ERR_TOO_LARGE, "too many angles for the angular-covariance kernel");

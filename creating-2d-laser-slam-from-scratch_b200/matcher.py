@@ -60,6 +60,7 @@ def lib():
     L.b2s_matcher_get_response_sums.argtypes = [vp, C.c_int, ip, ip]
     L.b2s_matcher_last_timing.argtypes = [vp, dp]
     L.b2s_matcher_last_stats.argtypes = [vp, dp]
+    L.b2s_matcher_last_prune_stats.argtypes = [vp, dp]
     L.b2s_matcher_sync.argtypes = [vp]
     L.b2s_matcher_set_kernel.argtypes = [vp, C.c_int]
     _lib = L
@@ -254,6 +255,12 @@ class ScanMatcher:
         out = np.zeros(4)
         check(self.L.b2s_matcher_last_stats(self.h, _d(out)))
         return dict(empty_window_frac=out[0], path=int(out[1]), candidates=int(out[2]), beams=int(out[3]))
+
+    def last_prune_stats(self):
+        """Angle pruning of the last correlate_scan: fraction and number of (match, angle) pairs swept."""
+        out = np.zeros(2)
+        check(self.L.b2s_matcher_last_prune_stats(self.h, _d(out)))
+        return dict(kept_frac=out[0], swept=int(out[1]))
 
     def sync(self):
         check(self.L.b2s_matcher_sync(self.h))

@@ -198,19 +198,28 @@ b2s_status b2s_matcher_correlate_scan_split(b2s_matcher *m, void *nccl_comm, int
                                             const b2s_search *search, b2s_match_result *results);
 /* ms of its last call: all-reduce(best), all-reduce(plane + status), all-reduce(tie sums), sweep end -> results */
 b2s_status b2s_matcher_last_split_timing(b2s_matcher *m, double out[4]);
+/* The whole integer response volume of the last sweep.  After a pruned sweep (b2s_matcher_last_prune_stats) the first
+ * call sweeps every angle once more from the lookup lists the handle still holds. */
 b2s_status b2s_matcher_get_response_sums(b2s_matcher *m, int b, int32_t *out, int32_t dims[3]);
 
 /* Device time (ms, CUDA events on the handle's stream) of the stages of the LAST correlate_scan call:
- * out[0] = offsets/LUT, out[1] = response sweep, out[2] = reduce (max / tie-average / covariance),
+ * out[0] = offsets/LUT, out[1] = response sweep (with the angle-pruning bound and select kernel when it runs),
+ * out[2] = reduce (max / tie-average / covariance),
  * out[3] = number of sweep kernel launches. */
 b2s_status b2s_matcher_last_timing(b2s_matcher *m, double out[4]);
 /* Statistics of the LAST correlate_scan call: out[0] = fraction of (beam, angle) windows the window kernel dropped
  * because every cell of the nY x nX window lies in empty 4x4 blocks of the grid (they add 0 to every candidate, so
  * results are unchanged); out[1] = sweep path (1 generic, 2 window); out[2] = candidates per match; out[3] = beams. */
 b2s_status b2s_matcher_last_stats(b2s_matcher *m, double out[4]);
+/* Angle pruning of the LAST correlate_scan call: out[0] = fraction of (match, angle) pairs the window kernel swept,
+ * out[1] = number of (match, angle) pairs swept.  A coarse-stage, stride-1 search of at most 32 x 32 cells whose grid
+ * fits shared memory first bounds every (angle, 4x4 candidate block) from a max-pooled grid and sweeps only the angles
+ * that can hold the best response, a tie or a cell the covariance reads; results are unchanged.  Without pruning
+ * out = {1, batch x angles}. */
+b2s_status b2s_matcher_last_prune_stats(b2s_matcher *m, double out[2]);
 b2s_status b2s_matcher_sync(b2s_matcher *m);
 /* 0 = automatic, 1 = force the generic global-memory gather kernel, 2 = force the shared-memory window kernel,
- * 3 = window kernel without dropping empty windows (every beam is swept) */
+ * 3 = window kernel without dropping empty windows and without angle pruning (every beam and every angle is swept) */
 b2s_status b2s_matcher_set_kernel(b2s_matcher *m, int which);
 
 /* ---------------------------------------------------------------- lesson6 front end: karto::Mapper / MapperGraph
